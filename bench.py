@@ -2,6 +2,7 @@
 """bench.py -- RNN-T loss+grad throughput on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5mb]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: loss + dense gradient
 w.r.t. log_probs for all lattices of the batch (what the reference's forward call produces,
@@ -17,6 +18,12 @@ pytorch_binding/benchmark.py:36-43), log_softmax excluded.
              reads + 4*N*(U-1) + 12*N) / measured step time, against MEASURED_PEAKS.json hbm_gbs.
   cpu_baseline  the CPU oracle port (oracle/rnnt_oracle.c, f32 flavour, OpenMP over lattices) timed on
              this box's host cores on a bounded sample of the same workload (rank 0, N=1 only).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned to the caller as
+float32 .npy files: DIR/loss.npy (the reduced loss) and DIR/grad.npy (the gradient w.r.t. the step's input); an
+output of more than 8M elements is written as a fixed sample of 8M of them (flat positions drawn with seed 0,
+ascending), so at most 64 MB in all.  The inputs are seeded: two builds run with the same arguments can be
+compared file by file.
 
 Multi-GPU (launched by torchrun): every rank runs the same per-GPU workload on its own shard
 (weak scaling, no data-path collective) and the scalar loss is all-reduced over NCCL each step.
@@ -203,6 +210,18 @@ def rotation(per_set_bytes):
     return int(max(2, min(6, (700e6 // per_set_bytes) + 1))) if per_set_bytes < 4e9 else 1
 
 
+def dump_outputs(dirname, outputs, max_elems=8 << 20):
+    """--dump-outputs: every tensor of `outputs` as dirname/<name>.npy in float32, a fixed sample of max_elems
+    elements (flat positions from seed 0, ascending) when it is larger."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.detach()
+        if a.numel() > max_elems:
+            idx = torch.randint(a.numel(), (max_elems,), generator=torch.Generator().manual_seed(0)).sort().values
+            a = a.reshape(-1)[idx.to(a.device)]
+        np.save(os.path.join(dirname, name + ".npy"), a.float().cpu().numpy())
+
+
 def timed(fn, steps, world, dist, dev, after=None):
     """CUDA events around exactly `steps` calls (+ `after()`, e.g. waiting for the last in-flight all-reduce), barrier +
     synchronize on both sides, max over ranks -> ms."""
@@ -239,7 +258,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="time the eager python API instead of CUDA-graph replays")
     ap.add_argument("--no-c5", action="store_true", help="skip the cfg-5 block of multi-GPU runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and the gradient of the last timed step to DIR/*.npy (float32; gradients "
+                         "of more than 8M elements as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -345,14 +369,21 @@ def main():
             g.replay()
             reduce_async(loss)
     else:
+        eager_loss = [None]
+
         def step(i):
-            reduce_async(api_step(sets[i % R]))
+            eager_loss[0] = api_step(sets[i % R])
+            reduce_async(eager_loss[0])
 
     for i in range(args.warmup):
         step(i)
     drain()
     n0 = w._C.launch_count()
     ms = timed(lambda i: step(args.warmup + i), args.steps, world, dist, dev, after=drain)
+    if args.dump_outputs and rank == 0:
+        last = (args.warmup + args.steps - 1) % R
+        dump_outputs(args.dump_outputs, {"loss": graphs[last][1] if graphs is not None else eager_loss[0],
+                                         "grad": sets[last][0].grad})
     launches = (launches_per_step * args.steps) if graphs is not None else int(w._C.launch_count() - n0)
     ms_per_step = ms / args.steps
     value = N * world * args.steps / (ms * 1e-3)

@@ -11,6 +11,7 @@ __init__.py:57-143 (python-level gather / average_frames / reduction).
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -20,15 +21,22 @@ _lib = None
 
 
 def build(force=False):
-    """gcc -> oracle/_build/librnnt_oracle.so (rebuilt when a source is newer)."""
+    """gcc -> oracle/_build/librnnt_oracle.so (rebuilt when a source is newer); into a fresh temporary
+    directory instead when oracle/ cannot be written (a read-only checkout)."""
     srcs = [os.path.join(_HERE, f) for f in ("rnnt_oracle.c", "rnnt_oracle_body.inc")]
-    os.makedirs(os.path.dirname(_LIB_PATH), exist_ok=True)
     stale = force or not os.path.exists(_LIB_PATH) or any(
         os.path.getmtime(s) > os.path.getmtime(_LIB_PATH) for s in srcs)
-    if stale:
-        subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-fopenmp", "-o", _LIB_PATH,
-                               srcs[0], "-lm"])
-    return _LIB_PATH
+    if not stale:
+        return _LIB_PATH
+    out = _LIB_PATH
+    try:
+        os.makedirs(os.path.dirname(_LIB_PATH), exist_ok=True)
+    except OSError:
+        pass
+    if not os.access(os.path.dirname(_LIB_PATH), os.W_OK):
+        out = os.path.join(tempfile.mkdtemp(prefix="rnnt_oracle_"), os.path.basename(_LIB_PATH))
+    subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-fopenmp", "-o", out, srcs[0], "-lm"])
+    return out
 
 
 def lib():

@@ -1,5 +1,5 @@
-"""GPU, BASELINE.json's full sizes: size-independent properties of the domain + the compiled
-reference where it finishes in seconds.
+"""GPU, BASELINE.json's full sizes: size-independent properties of the domain + the reference kernels' recorded
+outputs (tests/common.py ReferenceOutputs) where the reference finishes in seconds.
 
 Properties (all follow from alpha/beta being a flow on the lattice, SURVEY.md section 0):
   * every anti-diagonal t+u = d < Tn+Un-2 carries total flow 1:  -sum_{t+u=d}(g_blank + g_label) == 1
@@ -14,6 +14,8 @@ import numpy as np
 import pytest
 import torch
 
+from tests.common import ReferenceOutputs
+
 pytestmark = pytest.mark.gpu
 
 
@@ -23,10 +25,9 @@ def w():
     return warp_rnnt_b200
 
 
-@pytest.fixture(scope="module")
-def ref():
-    from oracle import build_ref
-    return build_ref.load()
+@pytest.fixture
+def reference(request):
+    return ReferenceOutputs(request)
 
 
 def synth(N, T, U, V, seed, random_lengths=False):
@@ -72,25 +73,24 @@ def check_properties(xs, ys, xn, yn, costs, grads, flow_tol):
     assert per[~live].abs().max().item() <= flow_tol if (~live).any() else True
 
 
-def test_cfg2_full(w, ref):
+def test_cfg2_full(w, reference):
     xs, ys, xn, yn = synth(128, 150, 40, 28, seed=128)
     w.set_lse_mode("fast")
     cf, gf = w._C.rnnt_loss(xs, ys, xn, yn)
     check_properties(xs, ys, xn, yn, cf, gf, flow_tol=2e-3)
     w.set_lse_mode("exact")
     ce, ge = w._C.rnnt_loss(xs, ys, xn, yn)
-    if ref is not None:
-        cr, gr = ref.rnnt_loss(xs, ys, xn, yn)
-        assert torch.equal(ce, cr) and torch.equal(ge, gr)          # bit-identical at full size
-        # the opt-in fast LSE: fp32 noise against the reference (measured 1.2e-4 on one of 21.5M
-        # gradient elements -- the reference itself is 1.25e-4 from the fp64 oracle at this shape).
-        # This is why the library default is the exact flavour.
-        assert ((cf - cr).abs() / cr.abs()).max().item() <= 1e-5
-        assert (gf - gr).abs().max().item() <= 2.5e-4
+    args = (xs, ys, xn, yn)
+    reference.check("dense", (ce, ge), lambda ref: ref.rnnt_loss(*args), args)     # bit-identical at full size
+    # the opt-in fast LSE: fp32 noise against the reference (= ce, ge; measured 1.2e-4 on one of 21.5M
+    # gradient elements -- the reference itself is 1.25e-4 from the fp64 oracle at this shape).
+    # This is why the library default is the exact flavour.
+    assert ((cf - ce).abs() / ce.abs()).max().item() <= 1e-5
+    assert (gf - ge).abs().max().item() <= 2.5e-4
     w.set_lse_mode("auto")
 
 
-def test_cfg2_random_lengths_python_api(w, ref):
+def test_cfg2_random_lengths_python_api(w, reference):
     xs, ys, xn, yn = synth(128, 150, 40, 28, seed=7, random_lengths=True)
     w.set_lse_mode("exact")
     x = xs.clone().requires_grad_(True)
@@ -99,20 +99,18 @@ def test_cfg2_random_lengths_python_api(w, ref):
     costs, grads = w._C.rnnt_loss(xs, ys, xn, yn)
     assert torch.equal(x.grad, grads)                              # deferred emit == eager emit, bit for bit
     check_properties(xs, ys, xn, yn, costs, grads, flow_tol=2e-3)
-    if ref is not None:
-        cr, gr = ref.rnnt_loss(xs, ys, xn, yn)
-        assert torch.equal(costs, cr) and torch.equal(grads, gr)
+    args = (xs, ys, xn, yn)
+    reference.check("dense", (costs, grads), lambda ref: ref.rnnt_loss(*args), args)
     w.set_lse_mode("auto")
 
 
-def test_cfg3_full(w, ref):
+def test_cfg3_full(w, reference):
     xs, ys, xn, yn = synth(32, 150, 20, 5000, seed=32)
     w.set_lse_mode("exact")
     ce, ge = w._C.rnnt_loss(xs, ys, xn, yn)
     check_properties(xs, ys, xn, yn, ce, ge, flow_tol=2e-3)
-    if ref is not None:
-        cr, gr = ref.rnnt_loss(xs, ys, xn, yn)
-        assert torch.equal(ce, cr) and torch.equal(ge, gr)
+    args = (xs, ys, xn, yn)
+    reference.check("dense", (ce, ge), lambda ref: ref.rnnt_loss(*args), args)
     w.set_lse_mode("auto")
 
 
@@ -140,7 +138,7 @@ def test_cfg4_full_dense_and_compact(w):
     w.set_lse_mode("auto")
 
 
-def test_cfg5_microbatch_independence_and_64bit(w, ref):
+def test_cfg5_microbatch_independence_and_64bit(w, reference):
     """N=32 T=600 U=150 V=1024: 2.9e9 gradient elements (> 2^31, the reference's int idx4 overflows
     beyond 23 lattices, core.cu:22-24).  A batch must equal its sub-batches bit for bit."""
     N, T, U, V = 32, 600, 150, 1024
@@ -152,9 +150,7 @@ def test_cfg5_microbatch_independence_and_64bit(w, ref):
                                 yn[lo:hi].contiguous())
         assert torch.equal(costs[lo:hi], c2) and torch.equal(grads[lo:hi], g2)
         del c2, g2
-    if ref is not None:
-        k = 4                                                          # the reference on the last 4 lattices
-        cr, gr = ref.rnnt_loss(xs[N - k:].contiguous(), ys[N - k:].contiguous(), xn[N - k:].contiguous(),
-                               yn[N - k:].contiguous())
-        assert torch.equal(costs[N - k:], cr) and torch.equal(grads[N - k:], gr)
+    k = 4                                                              # the reference on the last 4 lattices
+    args = tuple(t[N - k:].contiguous() for t in (xs, ys, xn, yn))
+    reference.check("dense", (costs[N - k:], grads[N - k:]), lambda ref: ref.rnnt_loss(*args), args)
     w.set_lse_mode("auto")

@@ -1,7 +1,8 @@
 """GPU: rnnt_loss_from_logits (fused log_softmax + loss, SURVEY.md 8(f)1) against
   (1) the fp64 oracle (oracle.from_logits = log_softmax then the loss, differentiated through both),
   (2) torch.log_softmax + this library's rnnt_loss through autograd (same kernels, unfused),
-  (3) torch.log_softmax + the compiled reference through autograd.
+  (3) torch.log_softmax + the reference kernels through autograd (their recorded outputs, tests/common.py
+      ReferenceOutputs: this library's exact mode reproduces them bit for bit).
 
 Not bit-identical by construction (the normaliser is summed in another order than torch's): stated tolerances are
 costs |d|/|ref| <= 1e-5 and gradients max|d| <= 1e-4 + gtol(T,U) (values in [-(1+lambda), 1+lambda])."""
@@ -10,6 +11,7 @@ import pytest
 import torch
 
 from oracle import oracle
+from tests.common import ReferenceOutputs
 
 pytestmark = pytest.mark.gpu
 
@@ -24,10 +26,9 @@ def w():
     return warp_rnnt_b200
 
 
-@pytest.fixture(scope="module")
-def ref():
-    from oracle import build_ref
-    return build_ref.load()
+@pytest.fixture
+def reference(request):
+    return ReferenceOutputs(request)
 
 
 def make(N, T, U, V, seed, blank=0, scale=3.0):
@@ -76,7 +77,7 @@ def test_from_logits_vs_oracle(w, shape, mode):
 
 
 @pytest.mark.parametrize("shape", [(4, 150, 40, 28, 0, 0.0), (2, 60, 33, 50, 0, 0.25), (2, 30, 12, 1024, 0, 0.0)])
-def test_from_logits_vs_unfused_and_reference(w, ref, shape):
+def test_from_logits_vs_unfused_and_reference(w, reference, shape):
     N, T, U, V, blank, lam = shape
     x, ys, xn, yn = make(N, T, U, V, seed=11 + V, blank=blank)
     args = (cu(ys), cu(xn), cu(yn))
@@ -89,14 +90,18 @@ def test_from_logits_vs_unfused_and_reference(w, ref, shape):
     lu.backward()
     np.testing.assert_allclose(loss.item(), lu.item(), rtol=1e-5)
     assert (xt.grad - xu.grad).abs().max().item() <= 1e-4 / N
-    if ref is not None:
-        xr = cu(x).requires_grad_(True)
-        lp = torch.log_softmax(xr, -1)
-        costs, grads = ref.rnnt_loss(lp.detach().contiguous(), *args, blank=blank, fastemit_lambda=lam)
-        wgt = (1.0 / cu(xn).float() / N).view(-1, 1, 1, 1)
-        lp.backward(grads * wgt)
-        np.testing.assert_allclose(loss.item(), (costs / cu(xn).float()).mean().item(), rtol=1e-5)
-        assert (xt.grad - xr.grad).abs().max().item() <= 1e-4 / N
+    xr = cu(x).requires_grad_(True)
+    lp = torch.log_softmax(xr, -1)
+    lpd = lp.detach().contiguous()
+    w.set_lse_mode("exact")
+    costs, grads = w._C.rnnt_loss(lpd, *args, blank=blank, fastemit_lambda=lam)
+    reference.check("dense", (costs, grads), lambda ref: ref.rnnt_loss(lpd, *args, blank=blank, fastemit_lambda=lam),
+                    (lpd,) + args)
+    w.set_lse_mode("auto")
+    wgt = (1.0 / cu(xn).float() / N).view(-1, 1, 1, 1)
+    lp.backward(grads * wgt)
+    np.testing.assert_allclose(loss.item(), (costs / cu(xn).float()).mean().item(), rtol=1e-5)
+    assert (xt.grad - xr.grad).abs().max().item() <= 1e-4 / N
 
 
 def test_from_logits_no_grad_and_invariance(w):
