@@ -61,10 +61,6 @@ static int forced_path() {
     }();
     return path;
 }
-static bool want_fused(int N, int T, int U, FusedPlan *plan) {
-    if (forced_path() >= 2) return false;
-    return fused_plan(N, T, U, plan);
-}
 
 struct Workspace {
     float2 *pairs;
@@ -75,23 +71,28 @@ struct Workspace {
     size_t bytes;
 };
 
-static Workspace carve(void *base, int64_t cells, int N) {
+// Sections of a workspace.  The native entry points take all of them (rnnt_b200_workspace_bytes); the
+// reference-ABI shims leave out what their call does not use, e.g. alphas and betas, which their caller owns.
+enum : unsigned { kWsPairs = 1, kWsLattices = 2, kWsLL = 4, kWsBad = 8, kWsPrefix = 16, kWsAll = 31 };
+
+static Workspace carve(void *base, int64_t cells, int N, unsigned parts = kWsAll) {
     Workspace w;
     size_t off = 0;
-    auto take = [&](size_t bytes) {
+    auto take = [&](unsigned part, size_t bytes) {
+        if (!(parts & part)) return (void *)nullptr;
         void *p = base ? (void *)((char *)base + off) : nullptr;
         off += align_up(bytes, 256);
         return p;
     };
     const size_t c = (size_t)(cells > 0 ? cells : 0), n = (size_t)(N > 0 ? N : 0);
-    w.pairs = (float2 *)take(c * sizeof(float2));
-    w.alphas = (float *)take(c * sizeof(float));
-    w.betas = (float *)take(c * sizeof(float));
-    w.ll = (float *)take(2 * n * sizeof(float));
-    w.bad = (int *)take(n * sizeof(int));
-    w.mem_pref = (int64_t *)take(n * sizeof(int64_t));
-    w.lab_pref = (int64_t *)take(n * sizeof(int64_t));
-    w.totals = (int *)take(4 * sizeof(int));
+    w.pairs = (float2 *)take(kWsPairs, c * sizeof(float2));
+    w.alphas = (float *)take(kWsLattices, c * sizeof(float));
+    w.betas = (float *)take(kWsLattices, c * sizeof(float));
+    w.ll = (float *)take(kWsLL, 2 * n * sizeof(float));
+    w.bad = (int *)take(kWsBad, n * sizeof(int));
+    w.mem_pref = (int64_t *)take(kWsPrefix, n * sizeof(int64_t));
+    w.lab_pref = (int64_t *)take(kWsPrefix, n * sizeof(int64_t));
+    w.totals = (int *)take(kWsPrefix, 4 * sizeof(int));
     w.bytes = off;
     return w;
 }
@@ -102,6 +103,12 @@ static bool dense_args_ok(int N, int T, int U, int V) {
     if ((int64_t)N * T * U >= (int64_t)1 << 31) return false;   // cell ids are 32-bit in the emit kernel
     if (V >= (1 << 22)) return false;
     return true;
+}
+// (cells,2) float2 buffers must be 8-byte aligned; null passes
+static bool f2_aligned(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
+// A dense-layout call: its shape, its blank id, and its (cells,2) gradient buffer (if any) aligned.
+static bool dense_call_ok(int N, int T, int U, int V, int blank, const void *pair_grads = nullptr) {
+    return dense_args_ok(N, T, U, V) && blank >= 0 && blank < V && f2_aligned(pair_grads);
 }
 
 // Internal streams for the pipelined general path: one for gathers, one for emits, four
@@ -206,36 +213,42 @@ __global__ void k_lse_selfcheck(unsigned long long *counts) {
         }                                                               \
     } while (0)
 
-}  // namespace rnnt
-
-using namespace rnnt;
-
-// dense layout, log_probs / grads of 4-byte (f32) or 2-byte (bf16) elements
-static int loss_dense_any(void *stream, void *workspace, size_t workspace_bytes, const void *log_probs,
-                          const int *labels, const int *xn, const int *yn, float *costs, void *grads,
-                          const float *grad_scale, float *loss_sum, unsigned int *sync_counter, int N, int T,
-                          int U, int V, int blank, float fastemit_lambda, int lse_mode, int io_bf16) {
-    const size_t esz = io_bf16 ? 2 : 4;
-    auto lp_at = [&](int64_t cell0) { return (const void *)((const char *)log_probs + (size_t)cell0 * V * esz); };
-    auto g_at = [&](int64_t cell0) { return (void *)((char *)grads + (size_t)cell0 * V * esz); };
-    if (io_bf16 && !grads) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (!dense_args_ok(N, T, U, V) || blank < 0 || blank >= V) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (N == 0) return RNNT_STATUS_SUCCESS;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t cells = (int64_t)N * T * U;
-    FusedPlan plan;
-    if (want_fused(N, T, U, &plan)) {
-        RNNT_TRY(launch_fused(s, resolve_kind(lse_mode, false), plan, log_probs, labels, xn, yn, costs, grads, nullptr,
-                              grad_scale, N, T, U, V, blank, fastemit_lambda, 0, 1, nullptr, nullptr, nullptr, loss_sum,
-                              sync_counter, io_bf16),
-                 RNNT_STATUS_WARP_FAILED);
-        if (loss_sum && !sync_counter)                  // no counter: reduce in a second, tiny launch
-            RNNT_TRY(launch_loss_sum(s, costs, grad_scale, N, loss_sum), RNNT_STATUS_COSTS_FAILED);
-        return RNNT_STATUS_SUCCESS;
+// The general sequence over the scratch in `w`: gather (unless the input already is pairs), the wavefront (beta
+// only when no gradient is asked for), then the dense emit or the (cells,2) gradients.
+static int run_general(cudaStream_t s, const LossJob &j, const Workspace &w) {
+    const int compact = j.mem_pref != nullptr;
+    const Problem p = {j.xn, j.yn, j.mem_pref, j.lab_pref, j.N, compact ? 0 : j.T, compact ? 0 : j.U, compact};
+    const float2 *pairs = j.pairs_in ? static_cast<const float2 *>(j.lp) : w.pairs;
+    // without the guard, `bad` would only mark the lattices that are not L.ok, which every later kernel checks itself
+    int *bad = j.guard ? w.bad : nullptr;
+    if (!j.pairs_in)
+        RNNT_TRY(launch_gather(s, p, j.lp, j.labels, j.V, j.blank, w.pairs, j.loc, j.cells, j.io_bf16),
+                 RNNT_STATUS_GATHER_FAILED);
+    RNNT_TRY(launch_wavefront(s, j.kind, p, pairs, w.alphas, w.betas, w.ll, bad, j.costs, !j.grads && !j.pair_grads,
+                              j.guard, j.T, j.U),
+             RNNT_STATUS_WARP_FAILED);
+    if (j.grads) {
+        ExpandSrc src = {};
+        src.pairs = pairs; src.alphas = w.alphas; src.betas = w.betas; src.bad = bad;
+        src.scale = j.scale; src.labels = j.labels; src.fastemit_lambda = j.lam;
+        RNNT_TRY(launch_expand(s, p, src, j.grads, j.cells, j.V, j.blank, false, j.io_bf16),
+                 RNNT_STATUS_GRADS_BLANK_FAILED);
+    } else if (j.pair_grads) {
+        RNNT_TRY(launch_grads_pairs(s, p, pairs, w.alphas, w.betas, bad, j.lam, j.pair_grads, j.cells),
+                 RNNT_STATUS_GRADS_BLANK_FAILED);
     }
-    const Workspace w = carve(workspace, cells, N);
-    if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
-    const int kind = resolve_kind(lse_mode, false);
+    return RNNT_STATUS_SUCCESS;
+}
+
+// The general sequence of a dense job with gradients, pipelined.  Returns false, having launched nothing, when the
+// batch is not pipelined; else true with the status in *status.
+static bool run_pipelined(cudaStream_t s, const LossJob &j, const Workspace &w, int *status) {
+    const int N = j.N, T = j.T, U = j.U, V = j.V, blank = j.blank, io_bf16 = j.io_bf16;
+    const int64_t cells = j.cells;
+    const void *grads = j.grads;
+    const size_t esz = io_bf16 ? 2 : 4;
+    auto lp_at = [&](int64_t cell0) { return (const void *)((const char *)j.lp + (size_t)cell0 * V * esz); };
+    auto g_at = [&](int64_t cell0) { return (void *)((char *)j.grads + (size_t)cell0 * V * esz); };
     // Large batches of large lattices: software-pipeline lattice groups over internal streams so that the
     // latency-bound wavefront of group g overlaps the bandwidth-bound gather of g+1 and emit of g-1.
     // ... which only pays when the wavefront (a per-lattice latency chain of T+U-1 steps, ~0.45 us each, that does not
@@ -245,64 +258,88 @@ static int loss_dense_any(void *stream, void *workspace, size_t workspace_bytes,
     const int groups = (grads && N >= 8 && (int64_t)cells * V * 4 >= ((int64_t)512 << 20) && pipeline_enabled() &&
                         wave_us < 0.4 * emit_us)
                            ? (N >= 32 ? 8 : 4) : 1;
-    if (groups > 1) {
-        std::lock_guard<std::mutex> lock(g_pipe_mu);    // the pipeline's events are shared by all calls on this device
-        Pipeline *pl = get_pipeline_locked();
-        if (pl) {
-            int status = RNNT_STATUS_SUCCESS;
-            cudaEventRecord(pl->fork, s);
-            cudaStreamWaitEvent(pl->gather_s, pl->fork, 0);
-            cudaStreamWaitEvent(pl->expand_s, pl->fork, 0);
-            for (int i = 0; i < Pipeline::kWave; ++i) cudaStreamWaitEvent(pl->wave_s[i], pl->fork, 0);
-            for (int g = 0; g < groups && !status; ++g) {
-                const int n0 = (int)((int64_t)N * g / groups), n1 = (int)((int64_t)N * (g + 1) / groups);
-                const int ng = n1 - n0;
-                const int64_t c0 = (int64_t)n0 * T * U, cg = (int64_t)ng * T * U;
-                Problem p = {xn + n0, yn + n0, nullptr, nullptr, ng, T, U, 0};
-                const int *lab_g = labels + (int64_t)n0 * (U - 1);
-                cudaStream_t ws = pl->wave_s[g % Pipeline::kWave];
-                if (launch_gather(pl->gather_s, p, lp_at(c0), lab_g, V, blank, w.pairs + c0, nullptr, cg, io_bf16) != cudaSuccess)
-                    status = RNNT_STATUS_GATHER_FAILED;
-                cudaEventRecord(pl->gathered[g], pl->gather_s);
-                cudaStreamWaitEvent(ws, pl->gathered[g], 0);
-                if (!status && launch_wavefront(ws, kind, p, w.pairs + c0, w.alphas + c0, w.betas + c0, w.ll + 2 * n0,
-                                                w.bad + n0, costs + n0, 0, 1, T, U) != cudaSuccess)
-                    status = RNNT_STATUS_WARP_FAILED;
-                cudaEventRecord(pl->swept[g], ws);
-                cudaStreamWaitEvent(pl->expand_s, pl->swept[g], 0);
-                ExpandSrc src = {};
-                src.pairs = w.pairs + c0; src.alphas = w.alphas + c0; src.betas = w.betas + c0; src.bad = w.bad + n0;
-                src.scale = grad_scale ? grad_scale + n0 : nullptr; src.labels = lab_g; src.fastemit_lambda = fastemit_lambda;
-                if (!status && launch_expand(pl->expand_s, p, src, g_at(c0), cg, V, blank, true, io_bf16) != cudaSuccess)
-                    status = RNNT_STATUS_GRADS_BLANK_FAILED;
-            }
-            cudaEventRecord(pl->join[0], pl->gather_s);
-            cudaEventRecord(pl->join[1], pl->expand_s);
-            cudaStreamWaitEvent(s, pl->join[0], 0);
-            cudaStreamWaitEvent(s, pl->join[1], 0);
-            for (int i = 0; i < Pipeline::kWave; ++i) {
-                cudaEventRecord(pl->join[2 + i], pl->wave_s[i]);
-                cudaStreamWaitEvent(s, pl->join[2 + i], 0);
-            }
-            if (!status && loss_sum && launch_loss_sum(s, costs, grad_scale, N, loss_sum) != cudaSuccess)
-                status = RNNT_STATUS_COSTS_FAILED;
-            return status;
-        }
-    }
-    Problem p = {xn, yn, nullptr, nullptr, N, T, U, 0};
-    RNNT_TRY(launch_gather(s, p, log_probs, labels, V, blank, w.pairs, nullptr, cells, io_bf16), RNNT_STATUS_GATHER_FAILED);
-    RNNT_TRY(launch_wavefront(s, kind, p, w.pairs, w.alphas, w.betas, w.ll, w.bad, costs, grads == nullptr, 1, T, U),
-             RNNT_STATUS_WARP_FAILED);
-    if (grads) {
+    if (groups <= 1) return false;
+    std::lock_guard<std::mutex> lock(g_pipe_mu);    // the pipeline's events are shared by all calls on this device
+    Pipeline *pl = get_pipeline_locked();
+    if (!pl) return false;
+    *status = RNNT_STATUS_SUCCESS;
+    cudaEventRecord(pl->fork, s);
+    cudaStreamWaitEvent(pl->gather_s, pl->fork, 0);
+    cudaStreamWaitEvent(pl->expand_s, pl->fork, 0);
+    for (int i = 0; i < Pipeline::kWave; ++i) cudaStreamWaitEvent(pl->wave_s[i], pl->fork, 0);
+    for (int g = 0; g < groups && !*status; ++g) {
+        const int n0 = (int)((int64_t)N * g / groups), n1 = (int)((int64_t)N * (g + 1) / groups);
+        const int ng = n1 - n0;
+        const int64_t c0 = (int64_t)n0 * T * U, cg = (int64_t)ng * T * U;
+        Problem p = {j.xn + n0, j.yn + n0, nullptr, nullptr, ng, T, U, 0};
+        const int *lab_g = j.labels + (int64_t)n0 * (U - 1);
+        cudaStream_t ws = pl->wave_s[g % Pipeline::kWave];
+        if (launch_gather(pl->gather_s, p, lp_at(c0), lab_g, V, blank, w.pairs + c0, nullptr, cg, io_bf16) != cudaSuccess)
+            *status = RNNT_STATUS_GATHER_FAILED;
+        cudaEventRecord(pl->gathered[g], pl->gather_s);
+        cudaStreamWaitEvent(ws, pl->gathered[g], 0);
+        if (!*status && launch_wavefront(ws, j.kind, p, w.pairs + c0, w.alphas + c0, w.betas + c0, w.ll + 2 * n0,
+                                         w.bad + n0, j.costs + n0, 0, 1, T, U) != cudaSuccess)
+            *status = RNNT_STATUS_WARP_FAILED;
+        cudaEventRecord(pl->swept[g], ws);
+        cudaStreamWaitEvent(pl->expand_s, pl->swept[g], 0);
         ExpandSrc src = {};
-        src.pairs = w.pairs; src.alphas = w.alphas; src.betas = w.betas; src.bad = w.bad;
-        src.scale = grad_scale; src.labels = labels; src.fastemit_lambda = fastemit_lambda;
-        RNNT_TRY(launch_expand(s, p, src, grads, cells, V, blank, false, io_bf16), RNNT_STATUS_GRADS_BLANK_FAILED);
+        src.pairs = w.pairs + c0; src.alphas = w.alphas + c0; src.betas = w.betas + c0; src.bad = w.bad + n0;
+        src.scale = j.scale ? j.scale + n0 : nullptr; src.labels = lab_g; src.fastemit_lambda = j.lam;
+        if (!*status && launch_expand(pl->expand_s, p, src, g_at(c0), cg, V, blank, true, io_bf16) != cudaSuccess)
+            *status = RNNT_STATUS_GRADS_BLANK_FAILED;
     }
-    if (loss_sum) RNNT_TRY(launch_loss_sum(s, costs, grad_scale, N, loss_sum), RNNT_STATUS_COSTS_FAILED);
+    cudaEventRecord(pl->join[0], pl->gather_s);
+    cudaEventRecord(pl->join[1], pl->expand_s);
+    cudaStreamWaitEvent(s, pl->join[0], 0);
+    cudaStreamWaitEvent(s, pl->join[1], 0);
+    for (int i = 0; i < Pipeline::kWave; ++i) {
+        cudaEventRecord(pl->join[2 + i], pl->wave_s[i]);
+        cudaStreamWaitEvent(s, pl->join[2 + i], 0);
+    }
+    return true;
+}
+
+// A native entry point's job: the fused kernel when its plan takes the shape (never for a compact job without
+// length bounds, T = U = 0) and RNNT_B200_PATH does not force the general path; else the general sequence over the
+// caller's workspace, pipelined where that pays.  Then the loss sum: inside the fused kernel when a counter is
+// given, else one more launch.
+static int dispatch(cudaStream_t s, const LossJob &j, void *workspace, size_t workspace_bytes) {
+    FusedPlan plan;
+    const bool fused = forced_path() < 2 && fused_plan(j.N, j.T, j.U, &plan);
+    if (fused) {
+        RNNT_TRY(launch_fused(s, j, plan), RNNT_STATUS_WARP_FAILED);
+    } else {
+        const Workspace w = carve(workspace, j.cells, j.N);
+        if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
+        int status;
+        if (!run_pipelined(s, j, w, &status)) status = run_general(s, j, w);
+        if (status) return status;
+    }
+    if (j.loss_sum && !(fused && j.sync_counter))
+        RNNT_TRY(launch_loss_sum(s, j.costs, j.scale, j.N, j.loss_sum), RNNT_STATUS_COSTS_FAILED);
     return RNNT_STATUS_SUCCESS;
 }
 
+}  // namespace rnnt
+
+using namespace rnnt;
+
+// dense layout, log_probs / grads of 4-byte (f32) or 2-byte (bf16) elements
+static int loss_dense_any(void *stream, void *workspace, size_t workspace_bytes, const void *log_probs,
+                          const int *labels, const int *xn, const int *yn, float *costs, void *grads,
+                          const float *grad_scale, float *loss_sum, unsigned int *sync_counter, int N, int T,
+                          int U, int V, int blank, float fastemit_lambda, int lse_mode, int io_bf16) {
+    if (io_bf16 && !grads) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (!dense_call_ok(N, T, U, V, blank)) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (N == 0) return RNNT_STATUS_SUCCESS;
+    LossJob j = {};
+    j.lp = log_probs; j.labels = labels; j.xn = xn; j.yn = yn; j.io_bf16 = io_bf16;
+    j.N = N; j.T = T; j.U = U; j.V = V; j.blank = blank; j.cells = (int64_t)N * T * U;
+    j.kind = resolve_kind(lse_mode, false); j.guard = 1; j.lam = fastemit_lambda;
+    j.costs = costs; j.grads = grads; j.scale = grad_scale; j.loss_sum = loss_sum; j.sync_counter = sync_counter;
+    return dispatch((cudaStream_t)stream, j, workspace, workspace_bytes);
+}
 
 extern "C" {
 
@@ -382,99 +419,49 @@ int rnnt_b200_rescale(void *stream, void *grads, const float *grad_out, int grad
 int rnnt_b200_loss_pairs(void *stream, void *workspace, size_t workspace_bytes, const float *pairs, const int *xn,
                          const int *yn, float *costs, float *pair_grads, int N, int T, int U,
                          float fastemit_lambda, int lse_mode) {
-    if (!dense_args_ok(N, T, U, 2)) return RNNT_STATUS_INVALID_ARGUMENT;
-    if ((reinterpret_cast<uintptr_t>(pairs) & 7u) || (reinterpret_cast<uintptr_t>(pair_grads) & 7u))
-        return RNNT_STATUS_INVALID_ARGUMENT;
+    if (!dense_call_ok(N, T, U, 2, 0, pair_grads) || !f2_aligned(pairs)) return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0) return RNNT_STATUS_SUCCESS;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t cells = (int64_t)N * T * U;
-    FusedPlan plan;
-    if (want_fused(N, T, U, &plan)) {
-        RNNT_TRY(launch_fused(s, resolve_kind(lse_mode, false), plan, pairs, nullptr, xn, yn, costs, nullptr,
-                              reinterpret_cast<float2 *>(pair_grads), nullptr, N, T, U, 2, 0, fastemit_lambda, 1, 1),
-                 RNNT_STATUS_WARP_FAILED);
-        return RNNT_STATUS_SUCCESS;
-    }
-    const Workspace w = carve(workspace, cells, N);
-    if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
-    Problem p = {xn, yn, nullptr, nullptr, N, T, U, 0};
-    const float2 *pr = reinterpret_cast<const float2 *>(pairs);
-    RNNT_TRY(launch_wavefront(s, resolve_kind(lse_mode, false), p, pr, w.alphas, w.betas, w.ll, w.bad, costs,
-                              pair_grads == nullptr, 1, T, U),
-             RNNT_STATUS_WARP_FAILED);
-    if (pair_grads)
-        RNNT_TRY(launch_grads_pairs(s, p, pr, w.alphas, w.betas, w.bad, fastemit_lambda,
-                                    reinterpret_cast<float2 *>(pair_grads), cells),
-                 RNNT_STATUS_GRADS_BLANK_FAILED);
-    return RNNT_STATUS_SUCCESS;
+    LossJob j = {};
+    j.lp = pairs; j.xn = xn; j.yn = yn; j.pairs_in = 1;
+    j.N = N; j.T = T; j.U = U; j.V = 2; j.blank = 0; j.cells = (int64_t)N * T * U;
+    j.kind = resolve_kind(lse_mode, false); j.guard = 1; j.lam = fastemit_lambda;
+    j.costs = costs; j.pair_grads = reinterpret_cast<float2 *>(pair_grads);
+    return dispatch((cudaStream_t)stream, j, workspace, workspace_bytes);
 }
 
 int rnnt_b200_gather_forward(void *stream, void *workspace, size_t workspace_bytes, const float *log_probs,
                              const int *labels, const int *xn, const int *yn, float *costs, float *pair_grads,
                              int N, int T, int U, int V, int blank, float fastemit_lambda, int lse_mode) {
-    if (!dense_args_ok(N, T, U, V) || blank < 0 || blank >= V) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (reinterpret_cast<uintptr_t>(pair_grads) & 7u) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (!dense_call_ok(N, T, U, V, blank, pair_grads)) return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0) return RNNT_STATUS_SUCCESS;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t cells = (int64_t)N * T * U;
-    FusedPlan plan;
-    if (want_fused(N, T, U, &plan)) {
-        RNNT_TRY(launch_fused(s, resolve_kind(lse_mode, false), plan, log_probs, labels, xn, yn, costs, nullptr,
-                              reinterpret_cast<float2 *>(pair_grads), nullptr, N, T, U, V, blank, fastemit_lambda, 0, 1),
-                 RNNT_STATUS_WARP_FAILED);
-        return RNNT_STATUS_SUCCESS;
-    }
-    const Workspace w = carve(workspace, cells, N);
-    if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
-    Problem p = {xn, yn, nullptr, nullptr, N, T, U, 0};
-    RNNT_TRY(launch_gather(s, p, log_probs, labels, V, blank, w.pairs, nullptr, cells), RNNT_STATUS_GATHER_FAILED);
-    RNNT_TRY(launch_wavefront(s, resolve_kind(lse_mode, false), p, w.pairs, w.alphas, w.betas, w.ll, w.bad, costs,
-                              pair_grads == nullptr, 1, T, U),
-             RNNT_STATUS_WARP_FAILED);
-    if (pair_grads)
-        RNNT_TRY(launch_grads_pairs(s, p, w.pairs, w.alphas, w.betas, w.bad, fastemit_lambda,
-                                    reinterpret_cast<float2 *>(pair_grads), cells),
-                 RNNT_STATUS_GRADS_BLANK_FAILED);
-    return RNNT_STATUS_SUCCESS;
+    LossJob j = {};
+    j.lp = log_probs; j.labels = labels; j.xn = xn; j.yn = yn;
+    j.N = N; j.T = T; j.U = U; j.V = V; j.blank = blank; j.cells = (int64_t)N * T * U;
+    j.kind = resolve_kind(lse_mode, false); j.guard = 1; j.lam = fastemit_lambda;
+    j.costs = costs; j.pair_grads = reinterpret_cast<float2 *>(pair_grads);
+    return dispatch((cudaStream_t)stream, j, workspace, workspace_bytes);
 }
 
 int rnnt_b200_logits_forward(void *stream, void *workspace, size_t workspace_bytes, const float *logits,
                               const int *labels, const int *xn, const int *yn, float *costs, float *lse,
                               float *pair_grads, int N, int T, int U, int V, int blank, float fastemit_lambda,
                               int lse_mode) {
-    if (!dense_args_ok(N, T, U, V) || blank < 0 || blank >= V || !lse) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (reinterpret_cast<uintptr_t>(pair_grads) & 7u) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (!dense_call_ok(N, T, U, V, blank, pair_grads) || !lse) return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0) return RNNT_STATUS_SUCCESS;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t cells = (int64_t)N * T * U;
-    const Workspace w = carve(workspace, cells, N);
+    const Workspace w = carve(workspace, (int64_t)N * T * U, N);
     if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
     // one pass over the logits: normaliser per cell + the two normalised log-probs the recurrence needs
-    RNNT_TRY(launch_lse_pairs(s, logits, labels, N, T, U, V, blank, w.pairs, lse), RNNT_STATUS_GATHER_FAILED);
-    // the (cells,2) layout from here on: same kernels as rnnt_b200_loss_pairs
-    const int kind = resolve_kind(lse_mode, false);
-    FusedPlan plan;
-    if (want_fused(N, T, U, &plan)) {
-        RNNT_TRY(launch_fused(s, kind, plan, reinterpret_cast<const float *>(w.pairs), nullptr, xn, yn, costs, nullptr,
-                              reinterpret_cast<float2 *>(pair_grads), nullptr, N, T, U, 2, 0, fastemit_lambda, 1, 1),
-                 RNNT_STATUS_WARP_FAILED);
-        return RNNT_STATUS_SUCCESS;
-    }
-    Problem p = {xn, yn, nullptr, nullptr, N, T, U, 0};
-    RNNT_TRY(launch_wavefront(s, kind, p, w.pairs, w.alphas, w.betas, w.ll, w.bad, costs, pair_grads == nullptr, 1, T, U),
-             RNNT_STATUS_WARP_FAILED);
-    if (pair_grads)
-        RNNT_TRY(launch_grads_pairs(s, p, w.pairs, w.alphas, w.betas, w.bad, fastemit_lambda,
-                                    reinterpret_cast<float2 *>(pair_grads), cells),
-                 RNNT_STATUS_GRADS_BLANK_FAILED);
-    return RNNT_STATUS_SUCCESS;
+    RNNT_TRY(launch_lse_pairs((cudaStream_t)stream, logits, labels, N, T, U, V, blank, w.pairs, lse),
+             RNNT_STATUS_GATHER_FAILED);
+    // the (cells,2) layout from here on: the job of rnnt_b200_loss_pairs over the workspace's pairs
+    return rnnt_b200_loss_pairs(stream, workspace, workspace_bytes, reinterpret_cast<const float *>(w.pairs), xn, yn,
+                                costs, pair_grads, N, T, U, fastemit_lambda, lse_mode);
 }
 
 int rnnt_b200_logits_backward(void *stream, const float *logits, const float *lse, const float *pair_grads,
                               const int *labels, const float *grad_out, float *out, int N, int T, int U, int V,
                               int blank) {
-    if (!dense_args_ok(N, T, U, V) || blank < 0 || blank >= V) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (reinterpret_cast<uintptr_t>(pair_grads) & 7u) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (!dense_call_ok(N, T, U, V, blank, pair_grads)) return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0) return RNNT_STATUS_SUCCESS;
     RNNT_TRY(launch_expand_logits((cudaStream_t)stream, logits, lse, reinterpret_cast<const float2 *>(pair_grads), labels,
                                   grad_out, out, N, T, U, V, blank),
@@ -484,8 +471,7 @@ int rnnt_b200_logits_backward(void *stream, const float *logits, const float *ls
 
 int rnnt_b200_gather_backward(void *stream, const float *pair_grads, const int *labels, const float *grad_out,
                               float *out, int N, int T, int U, int V, int blank, int accumulate, const int *yn) {
-    if (!dense_args_ok(N, T, U, V) || blank < 0 || blank >= V) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (reinterpret_cast<uintptr_t>(pair_grads) & 7u) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (!dense_call_ok(N, T, U, V, blank, pair_grads)) return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0) return RNNT_STATUS_SUCCESS;
     Problem p = {nullptr, yn, nullptr, nullptr, N, T, U, 0};     // yn (optional): which labels are real
     ExpandSrc src = {};
@@ -502,34 +488,21 @@ int rnnt_b200_compact_forward(void *stream, void *workspace, size_t workspace_by
                               const int *xn, const int *yn, float *costs, float *pair_grads, int64_t *loc,
                               int *totals, int64_t STU, int N, int V, int blank, float fastemit_lambda,
                               int lse_mode, int max_T, int max_U) {
-    if (N < 0 || STU < 0 || V < 1 || V >= (1 << 22) || blank < 0 || blank >= V) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (reinterpret_cast<uintptr_t>(pair_grads) & 7u) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (N < 0 || STU < 0 || V < 1 || V >= (1 << 22) || blank < 0 || blank >= V || !f2_aligned(pair_grads))
+        return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0) return RNNT_STATUS_SUCCESS;
     cudaStream_t s = (cudaStream_t)stream;
     const Workspace w = carve(workspace, STU, N);
     if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
     RNNT_TRY(launch_prefix(s, xn, yn, N, w.mem_pref, w.lab_pref, totals ? totals : w.totals), RNNT_STATUS_GATHER_FAILED);
-    Problem p = {xn, yn, w.mem_pref, w.lab_pref, N, 0, 0, 1};
-    FusedPlan fplan;
-    if (max_T > 0 && max_U > 0 && want_fused(N, max_T, max_U, &fplan)) {
-        // small lattices: gather + wavefront + (cells,2) gradients + loc in one launch (no mismatch guard in the
-        // compact reference, core_compact.cu:347-358)
-        RNNT_TRY(launch_fused(s, resolve_kind(lse_mode, true), fplan, xs, ys, xn, yn, costs, nullptr,
-                              reinterpret_cast<float2 *>(pair_grads), nullptr, N, max_T, max_U, V, blank,
-                              fastemit_lambda, 0, 0, w.mem_pref, w.lab_pref, loc),
-                 RNNT_STATUS_WARP_FAILED);
-        return RNNT_STATUS_SUCCESS;
-    }
-    RNNT_TRY(launch_gather(s, p, xs, ys, V, blank, w.pairs, loc, STU), RNNT_STATUS_GATHER_FAILED);
-    // no mismatch guard in the compact reference (core_compact.cu:347-358)
-    RNNT_TRY(launch_wavefront(s, resolve_kind(lse_mode, true), p, w.pairs, w.alphas, w.betas, w.ll, w.bad, costs,
-                              pair_grads == nullptr, 0, max_T, max_U),
-             RNNT_STATUS_WARP_FAILED);
-    if (pair_grads)
-        RNNT_TRY(launch_grads_pairs(s, p, w.pairs, w.alphas, w.betas, nullptr, fastemit_lambda,
-                                    reinterpret_cast<float2 *>(pair_grads), STU),
-                 RNNT_STATUS_GRADS_BLANK_FAILED);
-    return RNNT_STATUS_SUCCESS;
+    // the fused kernel (when max_T, max_U > 0 and it fits) also writes loc; no mismatch guard in the compact
+    // reference (core_compact.cu:347-358)
+    LossJob j = {};
+    j.lp = xs; j.labels = ys; j.xn = xn; j.yn = yn; j.mem_pref = w.mem_pref; j.lab_pref = w.lab_pref;
+    j.N = N; j.T = max_T; j.U = max_U; j.V = V; j.blank = blank; j.cells = STU;
+    j.kind = resolve_kind(lse_mode, true); j.guard = 0; j.lam = fastemit_lambda;
+    j.costs = costs; j.pair_grads = reinterpret_cast<float2 *>(pair_grads); j.loc = loc;
+    return dispatch(s, j, workspace, workspace_bytes);
 }
 
 int rnnt_b200_compact_totals(void *stream, const int *xn, const int *yn, int N, int64_t *scratch, int *totals) {
@@ -560,8 +533,8 @@ int rnnt_b200_joint_pack_backward(void *stream, const float *dx, const int *lf, 
 
 int rnnt_b200_compact_backward(void *stream, const float *grad_cost, const float *pair_grads, const int64_t *loc,
                                const int *cum_lens, float *out, int64_t STU, int N, int V, int blank) {
-    if (N < 0 || STU < 0 || V < 1 || V >= (1 << 22) || blank < 0 || blank >= V) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (reinterpret_cast<uintptr_t>(pair_grads) & 7u) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (N < 0 || STU < 0 || V < 1 || V >= (1 << 22) || blank < 0 || blank >= V || !f2_aligned(pair_grads))
+        return RNNT_STATUS_INVALID_ARGUMENT;
     if (N == 0 || STU == 0) return RNNT_STATUS_SUCCESS;
     Problem p = {nullptr, nullptr, nullptr, nullptr, N, 0, 0, 1};
     ExpandSrc src = {};
@@ -583,61 +556,53 @@ static void compat_die(const char *what, int status) {
     exit(-1);
 }
 
+// The `parts` of a workspace in one cudaMallocAsync block on `s`, or null; the caller frees it with cudaFreeAsync on `s`.
+static void *compat_scratch(cudaStream_t s, int64_t cells, int N, unsigned parts, Workspace *w) {
+    void *block = nullptr;
+    if (cudaMallocAsync(&block, carve(nullptr, cells, N, parts).bytes, s) != cudaSuccess) return nullptr;
+    *w = carve(block, cells, N, parts);
+    return block;
+}
+
+// The shims return alphas and betas, so they run the general sequence (never the fused kernel) with the caller's.
 int run_warp_rnnt(void *stream, unsigned int *counts, float *alphas, float *betas, const int *labels,
                   const float *log_probs, float *grads, float *costs, const int *xn, const int *yn, int N, int T,
                   int U, int V, int blank, float fastemit_lambda) {
     (void)counts;
-    if (!dense_args_ok(N, T, U, V) || blank < 0 || blank >= V) return RNNT_STATUS_WARP_FAILED;
+    if (!dense_call_ok(N, T, U, V, blank)) return RNNT_STATUS_WARP_FAILED;
     if (N == 0) return RNNT_STATUS_SUCCESS;
     cudaStream_t s = (cudaStream_t)stream;
-    const int64_t cells = (int64_t)N * T * U;
-    const size_t pair_bytes = align_up((size_t)cells * sizeof(float2), 256);
-    const size_t small = align_up(sizeof(float) * 2 * N, 256) + align_up(sizeof(int) * N, 256);
-    char *tmp = nullptr;
-    if (cudaMallocAsync((void **)&tmp, pair_bytes + small, s) != cudaSuccess) return RNNT_STATUS_WARP_FAILED;
-    float2 *pairs = (float2 *)tmp;
-    float *ll = (float *)(tmp + pair_bytes);
-    int *bad = (int *)(tmp + pair_bytes + align_up(sizeof(float) * 2 * N, 256));
-    Problem p = {xn, yn, nullptr, nullptr, N, T, U, 0};
-    int status = RNNT_STATUS_SUCCESS;
-    if (launch_gather(s, p, log_probs, labels, V, blank, pairs, nullptr, cells) != cudaSuccess)
-        status = RNNT_STATUS_WARP_FAILED;
-    if (!status && launch_wavefront(s, resolve_kind(RNNT_LSE_AUTO, false), p, pairs, alphas, betas, ll, bad, costs, 0,
-                                    1, T, U) != cudaSuccess)
-        status = RNNT_STATUS_WARP_FAILED;
-    if (!status) {
-        ExpandSrc src = {};
-        src.pairs = pairs; src.alphas = alphas; src.betas = betas; src.bad = bad;
-        src.labels = labels; src.fastemit_lambda = fastemit_lambda;
-        if (launch_expand(s, p, src, grads, cells, V, blank) != cudaSuccess) status = RNNT_STATUS_GRADS_BLANK_FAILED;
-    }
+    LossJob j = {};
+    j.lp = log_probs; j.labels = labels; j.xn = xn; j.yn = yn;
+    j.N = N; j.T = T; j.U = U; j.V = V; j.blank = blank; j.cells = (int64_t)N * T * U;
+    j.kind = resolve_kind(RNNT_LSE_AUTO, false); j.guard = 1; j.lam = fastemit_lambda;
+    j.costs = costs; j.grads = grads;
+    Workspace w;
+    void *tmp = compat_scratch(s, j.cells, N, kWsPairs | kWsLL | kWsBad, &w);
+    if (!tmp) return RNNT_STATUS_WARP_FAILED;
+    w.alphas = alphas; w.betas = betas;
+    const int status = run_general(s, j, w);
     cudaFreeAsync(tmp, s);
-    return status;
+    return status == RNNT_STATUS_GATHER_FAILED ? RNNT_STATUS_WARP_FAILED : status;   // the reference's statuses have no gather
 }
 
 int run_warp_rnnt_gather(void *stream, unsigned int *counts, float *alphas, float *betas, const float *log_probs,
                          float *grads, float *costs, const int *xn, const int *yn, int N, int T, int U,
                          float fastemit_lambda) {
     (void)counts;
-    if (!dense_args_ok(N, T, U, 2)) return RNNT_STATUS_WARP_FAILED;
+    if (!dense_call_ok(N, T, U, 2, 0)) return RNNT_STATUS_WARP_FAILED;
     if (N == 0) return RNNT_STATUS_SUCCESS;
     cudaStream_t s = (cudaStream_t)stream;
-    const int64_t cells = (int64_t)N * T * U;
-    const size_t llb = align_up(sizeof(float) * 2 * N, 256);
-    char *tmp = nullptr;
-    if (cudaMallocAsync((void **)&tmp, llb + align_up(sizeof(int) * N, 256), s) != cudaSuccess)
-        return RNNT_STATUS_WARP_FAILED;
-    float *ll = (float *)tmp;
-    int *bad = (int *)(tmp + llb);
-    Problem p = {xn, yn, nullptr, nullptr, N, T, U, 0};
-    const float2 *pr = reinterpret_cast<const float2 *>(log_probs);
-    int status = RNNT_STATUS_SUCCESS;
-    if (launch_wavefront(s, resolve_kind(RNNT_LSE_AUTO, false), p, pr, alphas, betas, ll, bad, costs, 0, 1, T, U) !=
-        cudaSuccess)
-        status = RNNT_STATUS_WARP_FAILED;
-    if (!status && launch_grads_pairs(s, p, pr, alphas, betas, bad, fastemit_lambda, reinterpret_cast<float2 *>(grads),
-                                      cells) != cudaSuccess)
-        status = RNNT_STATUS_GRADS_BLANK_FAILED;
+    LossJob j = {};
+    j.lp = log_probs; j.xn = xn; j.yn = yn; j.pairs_in = 1;
+    j.N = N; j.T = T; j.U = U; j.V = 2; j.blank = 0; j.cells = (int64_t)N * T * U;
+    j.kind = resolve_kind(RNNT_LSE_AUTO, false); j.guard = 1; j.lam = fastemit_lambda;
+    j.costs = costs; j.pair_grads = reinterpret_cast<float2 *>(grads);
+    Workspace w;
+    void *tmp = compat_scratch(s, j.cells, N, kWsLL | kWsBad, &w);
+    if (!tmp) return RNNT_STATUS_WARP_FAILED;
+    w.alphas = alphas; w.betas = betas;
+    const int status = run_general(s, j, w);
     cudaFreeAsync(tmp, s);
     return status;
 }
@@ -649,14 +614,12 @@ void run_gather_for_compact(const float *xs, const int *ys, const unsigned int *
     (void)memPref; (void)labelPref;   // recomputed on device in 64-bit
     if (N == 0) return;
     cudaStream_t s = 0;
-    const size_t pb = align_up(sizeof(int64_t) * N, 256);
-    char *tmp = nullptr;
-    if (cudaMallocAsync((void **)&tmp, 2 * pb + 256, s) != cudaSuccess) compat_die("rnnt loss gather for compact", RNNT_STATUS_GATHER_FAILED);
-    int64_t *mp = (int64_t *)tmp, *lp = (int64_t *)(tmp + pb);
-    int *totals = (int *)(tmp + 2 * pb);
+    Workspace w;
+    void *tmp = compat_scratch(s, 0, (int)N, kWsPrefix, &w);
+    if (!tmp) compat_die("rnnt loss gather for compact", RNNT_STATUS_GATHER_FAILED);
     const int *xi = (const int *)xn, *yi = (const int *)yn;
-    bool ok = launch_prefix(s, xi, yi, (int)N, mp, lp, totals) == cudaSuccess;
-    Problem p = {xi, yi, mp, lp, (int)N, 0, 0, 1};
+    bool ok = launch_prefix(s, xi, yi, (int)N, w.mem_pref, w.lab_pref, w.totals) == cudaSuccess;
+    Problem p = {xi, yi, w.mem_pref, w.lab_pref, (int)N, 0, 0, 1};
     ok = ok && launch_gather(s, p, xs, ys, (int)V, (int)blank, reinterpret_cast<float2 *>(gather_xs),
                              reinterpret_cast<int64_t *>(loc), (int64_t)N * T * U) == cudaSuccess;
     cudaFreeAsync(tmp, s);
@@ -670,22 +633,18 @@ void run_warp_rnnt_compact(unsigned int *counts, float *alphas, float *betas, co
     (void)counts; (void)memPref; (void)labelPref;
     if (N == 0) return;
     cudaStream_t s = 0;
-    const size_t pb = align_up(sizeof(int64_t) * N, 256);
-    const size_t llb = align_up(sizeof(float) * 2 * N, 256);
-    char *tmp = nullptr;
-    if (cudaMallocAsync((void **)&tmp, 2 * pb + llb + 256, s) != cudaSuccess) compat_die("rnnt loss compact betas", RNNT_STATUS_WARP_FAILED);
-    int64_t *mp = (int64_t *)tmp, *lp = (int64_t *)(tmp + pb);
-    float *ll = (float *)(tmp + 2 * pb);
-    int *totals = (int *)(tmp + 2 * pb + llb);
-    const int *xi = (const int *)xn, *yi = (const int *)yn;
-    bool ok = launch_prefix(s, xi, yi, (int)N, mp, lp, totals) == cudaSuccess;
-    Problem p = {xi, yi, mp, lp, (int)N, 0, 0, 1};
-    const float2 *pr = reinterpret_cast<const float2 *>(log_probs);
-    ok = ok && launch_wavefront(s, resolve_kind(RNNT_LSE_AUTO, true), p, pr, alphas, betas, ll, nullptr, costs,
-                                required_grad ? 0 : 1, 0, (int)T, (int)U) == cudaSuccess;
-    if (ok && required_grad)
-        ok = launch_grads_pairs(s, p, pr, alphas, betas, nullptr, fastemit_lambda, reinterpret_cast<float2 *>(grads),
-                                (int64_t)N * T * U) == cudaSuccess;
+    Workspace w;
+    void *tmp = compat_scratch(s, 0, (int)N, kWsLL | kWsPrefix, &w);
+    if (!tmp) compat_die("rnnt loss compact betas", RNNT_STATUS_WARP_FAILED);
+    w.alphas = alphas; w.betas = betas;
+    LossJob j = {};
+    j.lp = log_probs; j.xn = (const int *)xn; j.yn = (const int *)yn; j.mem_pref = w.mem_pref; j.lab_pref = w.lab_pref;
+    j.pairs_in = 1;
+    j.N = (int)N; j.T = (int)T; j.U = (int)U; j.V = 2; j.blank = 0; j.cells = (int64_t)N * T * U;
+    j.kind = resolve_kind(RNNT_LSE_AUTO, true); j.guard = 0; j.lam = fastemit_lambda;
+    j.costs = costs; j.pair_grads = required_grad ? reinterpret_cast<float2 *>(grads) : nullptr;
+    const bool ok = launch_prefix(s, j.xn, j.yn, j.N, w.mem_pref, w.lab_pref, w.totals) == cudaSuccess &&
+                    run_general(s, j, w) == RNNT_STATUS_SUCCESS;
     cudaFreeAsync(tmp, s);
     if (!ok) compat_die("rnnt loss compact", RNNT_STATUS_WARP_FAILED);
 }

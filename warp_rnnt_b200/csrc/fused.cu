@@ -896,18 +896,15 @@ static cudaError_t launch_fused_km(cudaStream_t s, const FusedArgs &a, size_t sm
     }
 }
 
-cudaError_t launch_fused(cudaStream_t s, int kind, const FusedPlan &plan, const void *lp, const int *labels,
-                         const int *xn, const int *yn, float *costs, void *grads, float2 *pair_grads,
-                         const float *scale, int N, int T, int U, int V, int blank, float lam, int pairs_in,
-                         int guard, const int64_t *mem_pref, const int64_t *lab_pref, int64_t *loc, float *loss_sum,
-                         unsigned *sync_counter, int io_bf16) {
+cudaError_t launch_fused(cudaStream_t s, const LossJob &j, const FusedPlan &plan) {
     FusedArgs a;
-    if (io_bf16 && (!grads || pairs_in || mem_pref)) return cudaErrorInvalidValue;   // bf16 i/o: dense gradients only
-    a.loss_sum = sync_counter ? loss_sum : nullptr; a.sync_counter = sync_counter;
-    a.mem_pref = mem_pref; a.lab_pref = lab_pref; a.loc = loc;
-    a.lp = lp; a.labels = labels; a.xn = xn; a.yn = yn; a.costs = costs; a.grads = grads; a.pair_grads = pair_grads;
-    a.scale = scale; a.N = N; a.T = T; a.U = U; a.V = V; a.blank = blank; a.lam = lam; a.pairs_in = pairs_in;
-    a.guard = guard; a.slices = (grads || pair_grads) ? plan.slices : 1; a.Wd = plan.W; a.nd = plan.ring;
+    if (j.io_bf16 && (!j.grads || j.pairs_in || j.mem_pref)) return cudaErrorInvalidValue;   // bf16 i/o: dense gradients only
+    a.loss_sum = j.sync_counter ? j.loss_sum : nullptr; a.sync_counter = j.sync_counter;
+    a.mem_pref = j.mem_pref; a.lab_pref = j.lab_pref; a.loc = j.loc;
+    a.lp = j.lp; a.labels = j.labels; a.xn = j.xn; a.yn = j.yn; a.costs = j.costs; a.grads = j.grads;
+    a.pair_grads = j.pair_grads; a.scale = j.scale; a.N = j.N; a.T = j.T; a.U = j.U; a.V = j.V; a.blank = j.blank;
+    a.lam = j.lam; a.pairs_in = j.pairs_in; a.guard = j.guard;
+    a.slices = (j.grads || j.pair_grads) ? plan.slices : 1; a.Wd = plan.W; a.nd = plan.ring;
     {
         static const int gw_raw = env_int("RNNT_B200_GATHER_WARPS", 0);   // tuning knob, in [1,14]
         const int gw_env = (gw_raw < 1 || gw_raw > kFusedThreads / 32 - 2) ? 0 : gw_raw;
@@ -915,7 +912,7 @@ cudaError_t launch_fused(cudaStream_t s, int kind, const FusedPlan &plan, const 
         // exact LSE: the wavefront outlasts the fill, so let every free warp gather and feed it sooner
         // (measured with the TMA fill: starting the fill only when the gather is done is best in both modes)
         a.gw = gw_env ? gw_env : kFusedThreads / 32 - 2;
-        if (!grads) a.gw = kFusedThreads / 32 - 2;      // nothing to fill: everyone gathers
+        if (!j.grads) a.gw = kFusedThreads / 32 - 2;      // nothing to fill: everyone gathers
     }
     a.zoff = (int)(plan.smem - kZeroBytes);
     // TMA row gather when a lattice row (U*V floats) is a 16-byte multiple at a 16-byte aligned address and
@@ -925,11 +922,11 @@ cudaError_t launch_fused(cudaStream_t s, int kind, const FusedPlan &plan, const 
     {
         static const bool want_tma = !env_is("RNNT_B200_GATHER", 'l');
         static const int nb_env = env_int("RNNT_B200_ROW_BUFS", 0);     // tuning knob: row buffers per gather warp (1 or 2)
-        const size_t row = (size_t)U * V * (io_bf16 ? 2 : sizeof(float));
+        const size_t row = (size_t)j.U * j.V * (j.io_bf16 ? 2 : sizeof(float));
         const size_t stride = (row + 127) / 128 * 128;
         // keep two CTAs per SM where the plan counted on them
         const size_t cap = (plan.smem <= 110 * 1024) ? (size_t)113 * 1024 : (size_t)kFusedMaxDynSmem;
-        if (want_tma && !pairs_in && (row % 16) == 0 && (reinterpret_cast<uintptr_t>(lp) % 16) == 0 && row <= 32 * 1024 &&
+        if (want_tma && !j.pairs_in && (row % 16) == 0 && (reinterpret_cast<uintptr_t>(j.lp) % 16) == 0 && row <= 32 * 1024 &&
             plan.smem + 4 * stride <= cap) {
             const int fit = (int)((cap - plan.smem) / stride);
             // two buffers per gather warp once at least 8 fit (the copy of the next row overlaps the picking of this one
@@ -951,9 +948,9 @@ cudaError_t launch_fused(cudaStream_t s, int kind, const FusedPlan &plan, const 
     }
     a.trace = g_fused_trace;
     { const GuardPoison gp = guard_poison(); a.poison_n = gp.n; a.poison_delta = gp.delta; }
-    const bool dense = grads != nullptr;
-    const int C = plan.nw;
-    if (io_bf16)
+    const bool dense = j.grads != nullptr;
+    const int C = plan.nw, kind = j.kind;
+    if (j.io_bf16)
         return kind == kFast ? launch_fused_km<kFast, 0, __nv_bfloat16>(s, a, smem, C)
                              : launch_fused_km<kExactDense, 0, __nv_bfloat16>(s, a, smem, C);
     if (kind == kFast)

@@ -52,17 +52,38 @@ cudaError_t launch_joint_pack(cudaStream_t s, const float *f, const float *g, co
 cudaError_t launch_joint_grads(cudaStream_t s, const float *dx, const int *lf, const int *lg, const int64_t *mem_pref,
                                float *df, float *dg, int N, int T, int U1, int H);
 
+// One loss call: its inputs, shape, numerics and outputs.  api.cu fills one per call and runs it either through
+// launch_fused or through the general sequence (gather, wavefront, gradient stage).
+struct LossJob {
+    // inputs
+    const void *lp;            // dense (N,T,U,V) log-probs, f32 or (io_bf16) bf16; pairs_in: (cells,2) f32
+    const int *labels;         // dense: (N,U-1); compact: (sum yn); pairs_in: unused
+    const int *xn, *yn;
+    const int64_t *mem_pref, *lab_pref;   // compact layout: first cell / first label of lattice n; dense: null
+    int pairs_in;              // lp is already the (cells,2) {blank, label} layout: no gather, V = 2, blank = 0
+    int io_bf16;               // lp and grads are bf16 (dense gradient only)
+    // shape
+    int N, T, U, V, blank;     // compact: T, U = upper bounds of the lengths, or 0 when unknown
+    int64_t cells;             // dense: N*T*U; compact: cells of the packed layout (or a bound on them)
+    // numerics
+    int kind;                  // LSE flavour (kExactDense, kExactCompact, kFast)
+    int guard;                 // forward/backward mismatch guard on
+    float lam;                 // FastEmit lambda
+    // outputs
+    float *costs;              // (N)
+    void *grads;               // dense gradient (N,T,U,V), or null
+    float2 *pair_grads;        // (cells,2) gradient, or null; with neither: loss only
+    const float *scale;        // (N) per-sample factor of the dense gradient and of loss_sum, or null
+    int64_t *loc;              // compact layout: label id per cell, written by the gather; or null
+    float *loss_sum;           // sum_n costs[n] * scale[n], or null
+    unsigned *sync_counter;    // with loss_sum: zeroed device counter that lets the fused kernel write the sum itself
+};
+
 // fused.cu -- single-kernel path for lattices that fit shared memory
 struct FusedPlan { int W, ring, nw, slices; size_t smem; };
 bool fused_plan(int N, int T, int U, FusedPlan *plan);
 void set_fused_trace(long long *buf);   // diagnostics: per-CTA phase stamps of k_fused (8 x clock64 per CTA)
-cudaError_t launch_fused(cudaStream_t s, int kind, const FusedPlan &plan, const void *lp, const int *labels,
-                         const int *xn, const int *yn, float *costs, void *grads, float2 *pair_grads,
-                         const float *scale, int N, int T, int U, int V, int blank, float lam, int pairs_in,
-                         int guard, const int64_t *mem_pref = nullptr, const int64_t *lab_pref = nullptr,
-                         int64_t *loc = nullptr,   // mem_pref != null: compact layout, T/U = max lengths
-                         float *loss_sum = nullptr, unsigned *sync_counter = nullptr,    // fused sum_n costs[n]*scale[n]
-                         int io_bf16 = 0);   // log_probs and the dense gradient are bf16 (dense MODE only)
+cudaError_t launch_fused(cudaStream_t s, const LossJob &job, const FusedPlan &plan);
 
 // expand.cu -- small helpers of the python-level API
 cudaError_t launch_loss_sum(cudaStream_t s, const float *costs, const float *scale, int N, float *loss_sum);
