@@ -182,6 +182,21 @@ int rnnt_b200_logits_backward(void *stream, const float *logits, const float *ls
                               const int *labels, const float *grad_out, float *out, int N, int T, int U, int V,
                               int blank);
 
+/* The same two calls with bfloat16 logits (N,T,U,V) and a bfloat16 logit gradient `out`; lse, costs, pair_grads and
+ * grad_out stay fp32.  Every bf16 value is converted exactly to fp32 and all arithmetic is the fp32 calls', in their
+ * order (the same elements are summed by the same lanes in the same order), so for bf16 logits x:
+ *   costs, lse and pair_grads are bit for bit those of rnnt_b200_logits_forward on x converted to fp32, in either LSE
+ *   mode, and out is that of rnnt_b200_logits_backward rounded once to bf16 (round to nearest even).
+ * Halves the bytes of the two dense passes.  An odd logits / out address returns RNNT_STATUS_INVALID_ARGUMENT
+ * (tests/test_gpu_logits_bf16.py). */
+int rnnt_b200_logits_forward_bf16(void *stream, void *workspace, size_t workspace_bytes, const void *logits_bf16,
+                                  const int *labels, const int *xn, const int *yn, float *costs, float *lse,
+                                  float *pair_grads, int N, int T, int U, int V, int blank, float fastemit_lambda,
+                                  int lse_mode);
+int rnnt_b200_logits_backward_bf16(void *stream, const void *logits_bf16, const float *lse, const float *pair_grads,
+                                   const int *labels, const float *grad_out, void *out_bf16, int N, int T, int U,
+                                   int V, int blank);
+
 /* Compact (ragged) layout.  xs (STU,V), ys (sum yn), STU = sum xn*(yn+1).
  * Replaces run_gather_for_compact + run_warp_rnnt_compact (core.h:41-55) and the host-side
  * prefix sums / .item() syncs of binding.cpp:132-158 (prefix sums are computed on device).

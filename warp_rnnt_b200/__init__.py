@@ -140,7 +140,12 @@ class RNNTLossFromLogits(torch.autograd.Function):
     The reference needs log-softmaxed input (README.md:59; its benchmark times ``F.log_softmax`` with the loss,
     benchmark.py:65): seven dense passes over (N,T,U,V) per step.  Here forward reads the logits once (per-cell
     normaliser + the two log-probs the recurrence needs) and keeps a (N,T,U,2) gradient; backward reads them once more
-    and writes d loss / d LOGITS, applying log_softmax's backward on the fly: three dense passes."""
+    and writes d loss / d LOGITS, applying log_softmax's backward on the fly: three dense passes.
+
+    Logits may be float32 or bfloat16 (e.g. a joint network run under ``torch.autocast(dtype=torch.bfloat16)``).  With
+    bfloat16 the two dense passes move half the bytes, the costs are float32, and the gradient handed to autograd is
+    bfloat16: all arithmetic is float32, and the results are bit for bit those of the float32 path on
+    ``logits.float()``, with the gradient rounded once to bfloat16."""
 
     @staticmethod
     def forward(ctx, logits, labels, frames_lengths, labels_lengths, blank=0, fastemit_lambda=0.0):
@@ -162,15 +167,16 @@ class RNNTLossFromLogits(torch.autograd.Function):
 def rnnt_loss_from_logits(logits, labels, frames_lengths, labels_lengths, average_frames=False, reduction="none",
                           blank=0, fastemit_lambda=0.0):
     """``rnnt_loss(log_softmax(logits, -1), ...)`` in three dense passes instead of seven; the gradient is w.r.t. the
-    LOGITS.  Dense (N,T,U,V) float32 layout; other arguments as in ``rnnt_loss``.  Agrees with
-    ``torch.log_softmax`` + the reference to 1e-5 (costs, relative) / 1e-4 (gradients), not bit for bit."""
+    LOGITS.  Dense (N,T,U,V) layout, float32 or bfloat16 logits (bfloat16: float32 costs and arithmetic, bfloat16
+    gradient, see ``RNNTLossFromLogits``); other arguments as in ``rnnt_loss``.  The loss is float32 for either dtype.
+    Agrees with ``torch.log_softmax`` + the reference to 1e-5 (costs, relative) / 1e-4 (gradients), not bit for bit."""
     assert average_frames is None or isinstance(average_frames, bool)
     assert reduction is None or reduction in ("none", "mean", "sum")
     assert isinstance(blank, int)
     assert not labels.requires_grad and not frames_lengths.requires_grad and not labels_lengths.requires_grad
     costs = RNNTLossFromLogits.apply(logits, labels, frames_lengths, labels_lengths, blank, fastemit_lambda)
     if average_frames:
-        costs = costs / frames_lengths.to(logits)
+        costs = costs / frames_lengths.to(torch.float32)       # not the logits' dtype: bf16 would round 257 frames to 256
     if reduction == "sum":
         return costs.sum()
     if reduction == "mean":

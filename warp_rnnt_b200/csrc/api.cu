@@ -341,6 +341,36 @@ static int loss_dense_any(void *stream, void *workspace, size_t workspace_bytes,
     return dispatch((cudaStream_t)stream, j, workspace, workspace_bytes);
 }
 
+// loss from logits of 4-byte (f32) or 2-byte (bf16) elements; lse, costs and pair gradients are f32 either way
+static int logits_forward_any(void *stream, void *workspace, size_t workspace_bytes, const void *logits,
+                              const int *labels, const int *xn, const int *yn, float *costs, float *lse,
+                              float *pair_grads, int N, int T, int U, int V, int blank, float fastemit_lambda,
+                              int lse_mode, int io_bf16) {
+    if (!dense_call_ok(N, T, U, V, blank, pair_grads) || !lse) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (N == 0) return RNNT_STATUS_SUCCESS;
+    const Workspace w = carve(workspace, (int64_t)N * T * U, N);
+    if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
+    // one pass over the logits: normaliser per cell + the two normalised log-probs the recurrence needs
+    RNNT_TRY(launch_lse_pairs((cudaStream_t)stream, logits, labels, N, T, U, V, blank, w.pairs, lse, io_bf16),
+             RNNT_STATUS_GATHER_FAILED);
+    // the (cells,2) layout from here on: the job of rnnt_b200_loss_pairs over the workspace's pairs
+    return rnnt_b200_loss_pairs(stream, workspace, workspace_bytes, reinterpret_cast<const float *>(w.pairs), xn, yn,
+                                costs, pair_grads, N, T, U, fastemit_lambda, lse_mode);
+}
+
+static int logits_backward_any(void *stream, const void *logits, const float *lse, const float *pair_grads,
+                               const int *labels, const float *grad_out, void *out, int N, int T, int U, int V,
+                               int blank, int io_bf16) {
+    if (!dense_call_ok(N, T, U, V, blank, pair_grads)) return RNNT_STATUS_INVALID_ARGUMENT;
+    if (N == 0) return RNNT_STATUS_SUCCESS;
+    RNNT_TRY(launch_expand_logits((cudaStream_t)stream, logits, lse, reinterpret_cast<const float2 *>(pair_grads), labels,
+                                  grad_out, out, N, T, U, V, blank, io_bf16),
+             RNNT_STATUS_GRADS_BLANK_FAILED);
+    return RNNT_STATUS_SUCCESS;
+}
+
+static bool bf16_aligned(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 1u) == 0; }
+
 extern "C" {
 
 const char *rnnt_b200_version(void) { return "0.1.0 (sm_100a)"; }
@@ -446,27 +476,30 @@ int rnnt_b200_logits_forward(void *stream, void *workspace, size_t workspace_byt
                               const int *labels, const int *xn, const int *yn, float *costs, float *lse,
                               float *pair_grads, int N, int T, int U, int V, int blank, float fastemit_lambda,
                               int lse_mode) {
-    if (!dense_call_ok(N, T, U, V, blank, pair_grads) || !lse) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (N == 0) return RNNT_STATUS_SUCCESS;
-    const Workspace w = carve(workspace, (int64_t)N * T * U, N);
-    if (!workspace || workspace_bytes < w.bytes) return RNNT_STATUS_WORKSPACE_TOO_SMALL;
-    // one pass over the logits: normaliser per cell + the two normalised log-probs the recurrence needs
-    RNNT_TRY(launch_lse_pairs((cudaStream_t)stream, logits, labels, N, T, U, V, blank, w.pairs, lse),
-             RNNT_STATUS_GATHER_FAILED);
-    // the (cells,2) layout from here on: the job of rnnt_b200_loss_pairs over the workspace's pairs
-    return rnnt_b200_loss_pairs(stream, workspace, workspace_bytes, reinterpret_cast<const float *>(w.pairs), xn, yn,
-                                costs, pair_grads, N, T, U, fastemit_lambda, lse_mode);
+    return logits_forward_any(stream, workspace, workspace_bytes, logits, labels, xn, yn, costs, lse, pair_grads, N, T,
+                              U, V, blank, fastemit_lambda, lse_mode, 0);
+}
+
+int rnnt_b200_logits_forward_bf16(void *stream, void *workspace, size_t workspace_bytes, const void *logits_bf16,
+                                  const int *labels, const int *xn, const int *yn, float *costs, float *lse,
+                                  float *pair_grads, int N, int T, int U, int V, int blank, float fastemit_lambda,
+                                  int lse_mode) {
+    if (!bf16_aligned(logits_bf16)) return RNNT_STATUS_INVALID_ARGUMENT;
+    return logits_forward_any(stream, workspace, workspace_bytes, logits_bf16, labels, xn, yn, costs, lse, pair_grads,
+                              N, T, U, V, blank, fastemit_lambda, lse_mode, 1);
 }
 
 int rnnt_b200_logits_backward(void *stream, const float *logits, const float *lse, const float *pair_grads,
                               const int *labels, const float *grad_out, float *out, int N, int T, int U, int V,
                               int blank) {
-    if (!dense_call_ok(N, T, U, V, blank, pair_grads)) return RNNT_STATUS_INVALID_ARGUMENT;
-    if (N == 0) return RNNT_STATUS_SUCCESS;
-    RNNT_TRY(launch_expand_logits((cudaStream_t)stream, logits, lse, reinterpret_cast<const float2 *>(pair_grads), labels,
-                                  grad_out, out, N, T, U, V, blank),
-             RNNT_STATUS_GRADS_BLANK_FAILED);
-    return RNNT_STATUS_SUCCESS;
+    return logits_backward_any(stream, logits, lse, pair_grads, labels, grad_out, out, N, T, U, V, blank, 0);
+}
+
+int rnnt_b200_logits_backward_bf16(void *stream, const void *logits_bf16, const float *lse, const float *pair_grads,
+                                   const int *labels, const float *grad_out, void *out_bf16, int N, int T, int U,
+                                   int V, int blank) {
+    if (!bf16_aligned(logits_bf16) || !bf16_aligned(out_bf16)) return RNNT_STATUS_INVALID_ARGUMENT;
+    return logits_backward_any(stream, logits_bf16, lse, pair_grads, labels, grad_out, out_bf16, N, T, U, V, blank, 1);
 }
 
 int rnnt_b200_gather_backward(void *stream, const float *pair_grads, const int *labels, const float *grad_out,

@@ -280,32 +280,43 @@ std::tuple<at::Tensor, at::Tensor> rnnt_gather_forward(const at::Tensor &xs, con
     return std::make_tuple(costs, pg);
 }
 
-// loss from un-normalised logits: (costs (N), lse (N,T,U), pair_grads (N,T,U,2) or empty)
+// loss from un-normalised logits, float32 or bfloat16: (costs (N), lse (N,T,U), pair_grads (N,T,U,2) or empty), all
+// three float32
 std::tuple<at::Tensor, at::Tensor, at::Tensor> rnnt_logits_forward(const at::Tensor &xs, const at::Tensor &ys,
                                                                    const at::Tensor &xn, const at::Tensor &yn,
                                                                    int blank, float fastemit_lambda, bool want_grads,
                                                                    int lse_mode) {
-    check4(xs, ys, xn, yn);
+    check4(xs, ys, xn, yn, true);
     check_dense_shapes(xs, ys, xn, yn);
     const c10::cuda::CUDAGuard guard(xs.device());
     const int64_t N = xs.size(0), T = xs.size(1), U = xs.size(2), V = xs.size(3);
     TORCH_CHECK(blank >= 0 && blank < V, "blank must be in [0, V)");
-    at::Tensor costs = at::empty({N}, xs.options());
-    at::Tensor lse = at::empty({N, T, U}, xs.options());
-    at::Tensor pg = want_grads ? at::empty({N, T, U, 2}, xs.options()) : at::empty({0}, xs.options());
+    const at::TensorOptions f32 = xs.options().dtype(at::kFloat);
+    at::Tensor costs = at::empty({N}, f32);
+    at::Tensor lse = at::empty({N, T, U}, f32);
+    at::Tensor pg = want_grads ? at::empty({N, T, U, 2}, f32) : at::empty({0}, f32);
     if (N == 0) return std::make_tuple(costs, lse, pg);
     at::Tensor ws = workspace_for(xs, N * T * U, N);
-    check_status(rnnt_b200_logits_forward(current_stream(xs), ws.data_ptr(), (size_t)ws.numel(), xs.data_ptr<float>(),
-                                          ys.data_ptr<int>(), xn.data_ptr<int>(), yn.data_ptr<int>(),
-                                          costs.data_ptr<float>(), lse.data_ptr<float>(),
-                                          want_grads ? pg.data_ptr<float>() : nullptr, (int)N, (int)T, (int)U, (int)V,
-                                          blank, fastemit_lambda, lse_mode));
+    float *pgp = want_grads ? pg.data_ptr<float>() : nullptr;
+    if (xs.scalar_type() == at::ScalarType::BFloat16)
+        check_status(rnnt_b200_logits_forward_bf16(current_stream(xs), ws.data_ptr(), (size_t)ws.numel(), xs.data_ptr(),
+                                                   ys.data_ptr<int>(), xn.data_ptr<int>(), yn.data_ptr<int>(),
+                                                   costs.data_ptr<float>(), lse.data_ptr<float>(), pgp, (int)N, (int)T,
+                                                   (int)U, (int)V, blank, fastemit_lambda, lse_mode));
+    else
+        check_status(rnnt_b200_logits_forward(current_stream(xs), ws.data_ptr(), (size_t)ws.numel(), xs.data_ptr<float>(),
+                                              ys.data_ptr<int>(), xn.data_ptr<int>(), yn.data_ptr<int>(),
+                                              costs.data_ptr<float>(), lse.data_ptr<float>(), pgp, (int)N, (int)T,
+                                              (int)U, (int)V, blank, fastemit_lambda, lse_mode));
     return std::make_tuple(costs, lse, pg);
 }
 
+// d loss / d logits, of the dtype of xs (float32 or bfloat16); lse, pair_grads and grad_out float32
 at::Tensor rnnt_logits_backward(const at::Tensor &xs, const at::Tensor &lse, const at::Tensor &pair_grads,
                                 const at::Tensor &ys, const at::Tensor &grad_out, int blank) {
-    TORCH_CHECK(xs.is_contiguous() && xs.scalar_type() == at::ScalarType::Float && xs.device().is_cuda() && xs.dim() == 4,
+    const bool bf16 = xs.scalar_type() == at::ScalarType::BFloat16;
+    TORCH_CHECK(xs.is_contiguous() && (xs.scalar_type() == at::ScalarType::Float || bf16) && xs.device().is_cuda() &&
+                    xs.dim() == 4,
                 "xs must be a contiguous CUDA Float tensor of shape (N, T, U, V)");
     const int64_t N = xs.size(0), T = xs.size(1), U = xs.size(2), V = xs.size(3);
     TORCH_CHECK(lse.is_contiguous() && lse.scalar_type() == at::ScalarType::Float && lse.device() == xs.device() &&
@@ -323,9 +334,15 @@ at::Tensor rnnt_logits_backward(const at::Tensor &xs, const at::Tensor &lse, con
     TORCH_CHECK(blank >= 0 && blank < V, "blank must be in [0, V)");
     const c10::cuda::CUDAGuard guard(xs.device());
     at::Tensor out = at::empty_like(xs);
-    check_status(rnnt_b200_logits_backward(current_stream(xs), xs.data_ptr<float>(), lse.data_ptr<float>(),
-                                           pair_grads.data_ptr<float>(), ys.data_ptr<int>(), grad_out.data_ptr<float>(),
-                                           out.data_ptr<float>(), (int)N, (int)T, (int)U, (int)V, blank));
+    if (bf16)
+        check_status(rnnt_b200_logits_backward_bf16(current_stream(xs), xs.data_ptr(), lse.data_ptr<float>(),
+                                                    pair_grads.data_ptr<float>(), ys.data_ptr<int>(),
+                                                    grad_out.data_ptr<float>(), out.data_ptr(), (int)N, (int)T, (int)U,
+                                                    (int)V, blank));
+    else
+        check_status(rnnt_b200_logits_backward(current_stream(xs), xs.data_ptr<float>(), lse.data_ptr<float>(),
+                                               pair_grads.data_ptr<float>(), ys.data_ptr<int>(), grad_out.data_ptr<float>(),
+                                               out.data_ptr<float>(), (int)N, (int)T, (int)U, (int)V, blank));
     return out;
 }
 

@@ -85,23 +85,12 @@ __device__ __forceinline__ void stage_row(const Problem &p, const ExpandSrc &src
     }
 }
 
-// MODE 0: dense layout, source = alpha/beta/pairs (forward)            label overrides blank
-// MODE 1: dense layout, source = pair grads (gather=True backward)     label adds to blank (scatter_add)
-// MODE 2: compact layout, source = pair grads + loc (compact backward) label written iff loc != blank
-// 16-byte streaming store of VEC output elements (4 floats or 8 bf16)
-__device__ __forceinline__ void st_vec(float *p, const float (&e)[4]) { st_cs_v4(p, make_float4(e[0], e[1], e[2], e[3])); }
-__device__ __forceinline__ void st_vec(__nv_bfloat16 *p, const float (&e)[8]) {
-    uint32_t w[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const __nv_bfloat162 h = __floats2bfloat162_rn(e[2 * k], e[2 * k + 1]);
-        w[k] = *reinterpret_cast<const uint32_t *>(&h);
-    }
-    asm volatile("st.global.cs.v4.b32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
-}
 __device__ __forceinline__ void st_one(float *p, float v) { st_cs(p, v); }
 __device__ __forceinline__ void st_one(__nv_bfloat16 *p, float v) { *p = __float2bfloat16_rn(v); }
 
+// MODE 0: dense layout, source = alpha/beta/pairs (forward)            label overrides blank
+// MODE 1: dense layout, source = pair grads (gather=True backward)     label adds to blank (scatter_add)
+// MODE 2: compact layout, source = pair grads + loc (compact backward) label written iff loc != blank
 // OUT: element type of the dense output (float; __nv_bfloat16 for the bf16 i/o forward, MODE 0)
 template <int MODE, typename OUT = float>
 __global__ void __launch_bounds__(kExpandThreads)
@@ -215,7 +204,7 @@ k_expand(Problem p, ExpandSrc src, OUT *__restrict__ out, int64_t cells, int V, 
                     if (++v == V) { v = 0; ++row; }
                 }
             }
-            st_vec(out + f, e);
+            st_cs_vec(out + f, e);            // 16 bytes: 4 floats or 8 bf16
         }
     }
 }

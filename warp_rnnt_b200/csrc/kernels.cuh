@@ -40,11 +40,12 @@ struct ExpandSrc {
 cudaError_t launch_expand(cudaStream_t s, const Problem &p, const ExpandSrc &src, void *out, int64_t cells,
                           int V, int blank, bool retire_early = false, int io_bf16 = 0);   // io_bf16: bf16 output (forward emit)
 
-// logits.cu -- loss from un-normalised logits (fused log_softmax forward / backward)
-cudaError_t launch_lse_pairs(cudaStream_t s, const float *x, const int *labels, int N, int T, int U, int V, int blank,
-                             float2 *pairs, float *lse);
-cudaError_t launch_expand_logits(cudaStream_t s, const float *x, const float *lse, const float2 *pg, const int *labels,
-                                 const float *grad_out, float *out, int N, int T, int U, int V, int blank);
+// logits.cu -- loss from un-normalised logits (fused log_softmax forward / backward); io_bf16: x (and out) bf16
+cudaError_t launch_lse_pairs(cudaStream_t s, const void *x, const int *labels, int N, int T, int U, int V, int blank,
+                             float2 *pairs, float *lse, int io_bf16 = 0);
+cudaError_t launch_expand_logits(cudaStream_t s, const void *x, const float *lse, const float2 *pg, const int *labels,
+                                 const float *grad_out, void *out, int N, int T, int U, int V, int blank,
+                                 int io_bf16 = 0);
 
 // joint.cu -- compact packing of the joint network's input (caller side of compact=True)
 cudaError_t launch_joint_pack(cudaStream_t s, const float *f, const float *g, const int *lf, const int *lg,

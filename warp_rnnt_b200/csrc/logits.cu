@@ -13,7 +13,8 @@
 //                    i.e. log_softmax's backward applied to the loss' (blank, label) gradient on the fly, times grad_out[n]
 //
 // three dense passes in total.  A label equal to blank: the two gradients add (what autograd through torch.gather /
-// log_softmax does).  Padded cells carry zero pair gradients and get exact zeros.
+// log_softmax does).  Padded cells carry zero pair gradients and get exact zeros.  Logits (and the logit gradient) are
+// float32 or bfloat16; lse, pairs and the pair gradients are float32 either way.
 #include "common.cuh"
 #include "kernels.cuh"
 
@@ -21,28 +22,47 @@ namespace rnnt {
 
 constexpr int kLogitThreads = 256;
 
+// Element types IO: float, or bf16 (bf16 logits in, bf16 logit gradient out).  Every bf16 value is converted exactly to
+// float on load and all arithmetic is the f32 path's, in the f32 path's order: both instantiations of a kernel give the
+// same lse / pairs bits on the same values, and the bf16 gradient is the f32 one rounded once (RNE) on the store.
+
+// the q-th 4-element vector of a 4-element-aligned row: one 16-byte (f32) or 8-byte (bf16) load
+__device__ __forceinline__ float4 ld4(const float *row, int q) { return __ldg(reinterpret_cast<const float4 *>(row) + q); }
+__device__ __forceinline__ float4 ld4(const __nv_bfloat16 *row, int q) {
+    const uint2 t = __ldg(reinterpret_cast<const uint2 *>(row) + q);
+    float4 a;
+    bf16x2_to_float(t.x, a.x, a.y);
+    bf16x2_to_float(t.y, a.z, a.w);
+    return a;
+}
+
+// iterations of the vec4 loop whose loads are issued ahead of their math: a bf16 lane loads 8 bytes per iteration,
+// half of what an f32 lane does, so it keeps four iterations in flight; f32 keeps its one 16-byte load per iteration.
+template <typename IO> constexpr int kLseIlp = sizeof(IO) == 2 ? 4 : 1;
+
 // SUB lanes cooperate on one cell (SUB in {1, 8, 32}); online max / sum so the row is read once.  VEC4: rows are whole
-// float4s at 16-byte aligned addresses -> the SUB lanes stride over float4s (V = 28: 7 of 8 lanes load one vector each,
-// a warp reads 4 consecutive rows = 448 contiguous bytes).
-template <int SUB, bool VEC4>
+// 4-element vectors at 4-element-aligned addresses -> the SUB lanes stride over vectors (V = 28: 7 of 8 lanes load one
+// vector each, a warp reads 4 consecutive rows = 448 contiguous bytes in f32).  Lane `sub` sums vectors sub, sub + SUB,
+// ... in that order for either element type.
+template <typename IO, int SUB, bool VEC4>
 __global__ void __launch_bounds__(kLogitThreads)
-k_lse_pairs(const float *__restrict__ x, const int *__restrict__ labels, int64_t cells, int V, int blank, int U,
+k_lse_pairs(const IO *__restrict__ x, const int *__restrict__ labels, int64_t cells, int V, int blank, int U,
             FastDiv divU, FastDiv divTU, float2 *__restrict__ pairs, float *__restrict__ lse_out) {
     const int sub = threadIdx.x % SUB;
     const int64_t per_block = kLogitThreads / SUB;
     for (int64_t base = (int64_t)blockIdx.x * per_block; base < cells; base += (int64_t)gridDim.x * per_block) {   // block-uniform trip count
         const int64_t cell = min(base + threadIdx.x / SUB, cells - 1);          // surplus groups redo the last cell (shuffles need every lane)
-        const float *row = x + cell * V;
+        const IO *row = x + cell * V;
         float m = -INFINITY, s = 0.0f;
         auto add = [&](float a) {
             if (a > m) { s = s * expf(m - a); m = a; }        // (m == -inf: s is 0, exp(-inf) = 0)
             s += expf(a - m);
         };
         if (VEC4 && (V >> 2) <= SUB) {
-            // the whole row is one float4 per lane: max first (shuffles only), then ONE exp per element -- the online
+            // the whole row is one vector per lane: max first (shuffles only), then ONE exp per element -- the online
             // merge below would spend two more exp per lane and shuffle round
             const bool has = sub < (V >> 2);
-            const float4 a = has ? __ldg(reinterpret_cast<const float4 *>(row) + sub) : make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
+            const float4 a = has ? ld4(row, sub) : make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
             m = fmaxf(fmaxf(a.x, a.y), fmaxf(a.z, a.w));
 #pragma unroll
             for (int o = SUB / 2; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
@@ -50,20 +70,30 @@ k_lse_pairs(const float *__restrict__ x, const int *__restrict__ labels, int64_t
 #pragma unroll
             for (int o = SUB / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
         } else if (VEC4) {
-            const float4 *row4 = reinterpret_cast<const float4 *>(row);
-            for (int q = sub; q < (V >> 2); q += SUB) {
-                const float4 a = __ldg(row4 + q);
+            auto add4 = [&](const float4 a) {
                 const float mx = fmaxf(fmaxf(a.x, a.y), fmaxf(a.z, a.w));
                 if (mx > m) { s = s * expf(m - mx); m = mx; }
                 s += (expf(a.x - m) + expf(a.y - m)) + (expf(a.z - m) + expf(a.w - m));
+            };
+            constexpr int ILP = kLseIlp<IO>;
+            int q0 = sub;
+            if constexpr (ILP > 1) {
+                for (; q0 + (ILP - 1) * SUB < (V >> 2); q0 += ILP * SUB) {
+                    float4 a[ILP];
+#pragma unroll
+                    for (int k = 0; k < ILP; ++k) a[k] = ld4(row, q0 + k * SUB);
+#pragma unroll
+                    for (int k = 0; k < ILP; ++k) add4(a[k]);
+                }
             }
+            for (int q = q0; q < (V >> 2); q += SUB) add4(ld4(row, q));
         } else if (SUB == 1) {
             // short unaligned rows: one thread per cell; neighbouring threads' rows share cache lines, so the pass over
             // v is served from L1 after the first touch
-            for (int v = 0; v < V; ++v) m = fmaxf(m, __ldg(row + v));
-            for (int v = 0; v < V; ++v) s += expf(__ldg(row + v) - m);
+            for (int v = 0; v < V; ++v) m = fmaxf(m, io_load<IO>(row + v));
+            for (int v = 0; v < V; ++v) s += expf(io_load<IO>(row + v) - m);
         } else {
-            for (int v = sub; v < V; v += SUB) add(__ldg(row + v));
+            for (int v = sub; v < V; v += SUB) add(io_load<IO>(row + v));
         }
         if (SUB > 1 && !(VEC4 && (V >> 2) <= SUB)) {
 #pragma unroll
@@ -80,25 +110,26 @@ k_lse_pairs(const float *__restrict__ x, const int *__restrict__ labels, int64_t
             divTU.divmod((uint32_t)cell, n, rem);
             divU.divmod(rem, t, u);
             const int lab = ((int)u < U - 1) ? labels[(int64_t)n * (U - 1) + u] : blank;
-            pairs[cell] = make_float2(__ldg(row + blank) - l, __ldg(row + lab) - l);
+            pairs[cell] = make_float2(io_load<IO>(row + blank) - l, io_load<IO>(row + lab) - l);
             lse_out[cell] = l;
         }
     }
 }
 
-// flat stream of the (cells, V) output in vectors of VEC floats (VEC = 4 when V % 4 == 0, 2 when V % 2 == 0, else 1):
-// a vector never straddles a row, so one (gb, gl, lse, label) fetch serves it.
-template <int VEC>
+// flat stream of the (cells, V) output in vectors of VEC elements (the widest of at most 16 bytes that divides V and
+// the alignment of both pointers): a vector never straddles a row, so one (gb, gl, lse, label) fetch serves it.  The
+// arithmetic is per element, so VEC does not change the values.
+template <typename IO, int VEC>
 __global__ void __launch_bounds__(kLogitThreads)
-k_expand_logits(const float *__restrict__ x, const float *__restrict__ lse, const float2 *__restrict__ pg,
-                const int *__restrict__ labels, const float *__restrict__ grad_out, float *__restrict__ out,
+k_expand_logits(const IO *__restrict__ x, const float *__restrict__ lse, const float2 *__restrict__ pg,
+                const int *__restrict__ labels, const float *__restrict__ grad_out, IO *__restrict__ out,
                 int64_t cells, int V, int blank, int U, FastDiv divU, FastDiv divTU, int64_t stride_rows,
                 int stride_v) {
     const int64_t total = cells * (int64_t)V;
     int64_t f = ((int64_t)blockIdx.x * kLogitThreads + threadIdx.x) * VEC;
     if (f >= total) return;
     // (row, v0) of the thread's vector: one 64-bit division here, then a running cursor (the grid stride is
-    // stride_rows whole rows + stride_v floats)
+    // stride_rows whole rows + stride_v elements)
     int64_t row = f / V;
     int v0 = (int)(f - row * V);
     const int64_t stride = stride_rows * V + stride_v;
@@ -117,15 +148,7 @@ k_expand_logits(const float *__restrict__ x, const float *__restrict__ lse, cons
             const float sc = grad_out ? grad_out[n] : 1.0f;
             const float l = lse[row], tot = q.x + q.y;
             float xv[VEC];
-            if (VEC == 4) {
-                const float4 t4 = __ldg(reinterpret_cast<const float4 *>(x + f));
-                xv[0] = t4.x; xv[1] = t4.y; xv[2 % VEC] = t4.z; xv[3 % VEC] = t4.w;
-            } else if (VEC == 2) {
-                const float2 t2 = __ldg(reinterpret_cast<const float2 *>(x + f));
-                xv[0] = t2.x; xv[1 % VEC] = t2.y;
-            } else {
-                xv[0] = __ldg(x + f);
-            }
+            ld_vec<VEC>(x + f, xv);
 #pragma unroll
             for (int k = 0; k < VEC; ++k) {
                 float gsel = (v0 + k == blank) ? q.x : 0.0f;
@@ -133,49 +156,75 @@ k_expand_logits(const float *__restrict__ x, const float *__restrict__ lse, cons
                 e[k] = (gsel - expf(xv[k] - l) * tot) * sc;
             }
         }
-        if (VEC == 4) st_cs_v4(out + f, make_float4(e[0], e[1 % VEC], e[2 % VEC], e[3 % VEC]));
-        else if (VEC == 2) st_cs_v2(out + f, make_float2(e[0], e[1 % VEC]));
-        else st_cs(out + f, e[0]);
+        st_cs_vec<VEC>(out + f, e);
     }
 }
 
-cudaError_t launch_lse_pairs(cudaStream_t s, const float *x, const int *labels, int N, int T, int U, int V, int blank,
-                             float2 *pairs, float *lse) {
-    const int64_t cells = (int64_t)N * T * U;
-    if (cells <= 0) return cudaSuccess;
-    const FastDiv divU((uint32_t)U), divTU((uint32_t)(T * U));
-    const int sms = sm_count(current_device());
-    const bool vec4 = (V % 4 == 0) && ((reinterpret_cast<uintptr_t>(x) & 15u) == 0);
-    const int sub = vec4 ? (V <= 32 ? 8 : 32) : (V <= 12 ? 1 : (V <= 512 ? 8 : 32));
-    const int64_t per_block = kLogitThreads / sub;
-    const int grid = (int)min((cells + per_block - 1) / per_block, (int64_t)sms * 16);
-#define RNNT_LSE_LAUNCH(SUB, VEC) k_lse_pairs<SUB, VEC><<<grid, kLogitThreads, 0, s>>>(x, labels, cells, V, blank, U, divU, divTU, pairs, lse)
+template <typename IO>
+static void lse_pairs_io(cudaStream_t s, int grid, bool vec4, int sub, const IO *x, const int *labels, int64_t cells,
+                         int V, int blank, int U, FastDiv divU, FastDiv divTU, float2 *pairs, float *lse) {
+#define RNNT_LSE_LAUNCH(SUB, VEC) k_lse_pairs<IO, SUB, VEC><<<grid, kLogitThreads, 0, s>>>(x, labels, cells, V, blank, U, divU, divTU, pairs, lse)
     if (vec4) { if (sub == 8) RNNT_LSE_LAUNCH(8, true); else RNNT_LSE_LAUNCH(32, true); }
     else if (sub == 1) RNNT_LSE_LAUNCH(1, false);
     else if (sub == 8) RNNT_LSE_LAUNCH(8, false);
     else RNNT_LSE_LAUNCH(32, false);
 #undef RNNT_LSE_LAUNCH
-    count_launch();
-    return cudaGetLastError();
 }
 
-cudaError_t launch_expand_logits(cudaStream_t s, const float *x, const float *lse, const float2 *pg, const int *labels,
-                                 const float *grad_out, float *out, int N, int T, int U, int V, int blank) {
+cudaError_t launch_lse_pairs(cudaStream_t s, const void *x, const int *labels, int N, int T, int U, int V, int blank,
+                             float2 *pairs, float *lse, int io_bf16) {
     const int64_t cells = (int64_t)N * T * U;
     if (cells <= 0) return cudaSuccess;
     const FastDiv divU((uint32_t)U), divTU((uint32_t)(T * U));
     const int sms = sm_count(current_device());
-    const bool al16 = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out)) & 15u) == 0;
-    const bool al8 = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out)) & 7u) == 0;
-    const int vec = (V % 4 == 0 && al16) ? 4 : ((V % 2 == 0 && al8) ? 2 : 1);
+    // variant chosen in elements, the same for both element types (it fixes which lane sums which elements)
+    const uintptr_t vec_bytes = 4 * (io_bf16 ? sizeof(__nv_bfloat16) : sizeof(float));
+    const bool vec4 = (V % 4 == 0) && ((reinterpret_cast<uintptr_t>(x) & (vec_bytes - 1)) == 0);
+    const int sub = vec4 ? (V <= 32 ? 8 : 32) : (V <= 12 ? 1 : (V <= 512 ? 8 : 32));
+    const int64_t per_block = kLogitThreads / sub;
+    const int grid = (int)min((cells + per_block - 1) / per_block, (int64_t)sms * 16);
+    if (io_bf16)
+        lse_pairs_io(s, grid, vec4, sub, static_cast<const __nv_bfloat16 *>(x), labels, cells, V, blank, U, divU, divTU, pairs, lse);
+    else
+        lse_pairs_io(s, grid, vec4, sub, static_cast<const float *>(x), labels, cells, V, blank, U, divU, divTU, pairs, lse);
+    count_launch();
+    return cudaGetLastError();
+}
+
+template <typename IO>
+static void expand_logits_io(cudaStream_t s, int grid, int vec, const IO *x, const float *lse, const float2 *pg,
+                             const int *labels, const float *grad_out, IO *out, int64_t cells, int V, int blank, int U,
+                             FastDiv divU, FastDiv divTU, int64_t srows, int sv) {
+#define RNNT_EXPAND_LAUNCH(VEC) k_expand_logits<IO, VEC><<<grid, kLogitThreads, 0, s>>>(x, lse, pg, labels, grad_out, out, cells, V, blank, U, divU, divTU, srows, sv)
+    if constexpr (sizeof(IO) == 2) { if (vec == 8) { RNNT_EXPAND_LAUNCH(8); return; } }
+    if (vec == 4) RNNT_EXPAND_LAUNCH(4);
+    else if (vec == 2) RNNT_EXPAND_LAUNCH(2);
+    else RNNT_EXPAND_LAUNCH(1);
+#undef RNNT_EXPAND_LAUNCH
+}
+
+cudaError_t launch_expand_logits(cudaStream_t s, const void *x, const float *lse, const float2 *pg, const int *labels,
+                                 const float *grad_out, void *out, int N, int T, int U, int V, int blank, int io_bf16) {
+    const int64_t cells = (int64_t)N * T * U;
+    if (cells <= 0) return cudaSuccess;
+    const FastDiv divU((uint32_t)U), divTU((uint32_t)(T * U));
+    const int sms = sm_count(current_device());
+    // the widest vector of at most 16 bytes that divides V and to which both pointers are aligned
+    const size_t esz = io_bf16 ? sizeof(__nv_bfloat16) : sizeof(float);
+    const uintptr_t addr = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(out);
+    int vec = (int)(16 / esz);
+    while (vec > 1 && (V % vec != 0 || (addr & (vec * esz - 1)) != 0)) vec >>= 1;
     const int64_t total = cells * (int64_t)V / vec;
     const int grid = (int)min((total + kLogitThreads - 1) / kLogitThreads, (int64_t)sms * 32);
     const int64_t stride = (int64_t)grid * kLogitThreads * vec;
     const int64_t srows = stride / V;
     const int sv = (int)(stride - srows * V);
-    if (vec == 4) k_expand_logits<4><<<grid, kLogitThreads, 0, s>>>(x, lse, pg, labels, grad_out, out, cells, V, blank, U, divU, divTU, srows, sv);
-    else if (vec == 2) k_expand_logits<2><<<grid, kLogitThreads, 0, s>>>(x, lse, pg, labels, grad_out, out, cells, V, blank, U, divU, divTU, srows, sv);
-    else k_expand_logits<1><<<grid, kLogitThreads, 0, s>>>(x, lse, pg, labels, grad_out, out, cells, V, blank, U, divU, divTU, srows, sv);
+    if (io_bf16)
+        expand_logits_io(s, grid, vec, static_cast<const __nv_bfloat16 *>(x), lse, pg, labels, grad_out,
+                         static_cast<__nv_bfloat16 *>(out), cells, V, blank, U, divU, divTU, srows, sv);
+    else
+        expand_logits_io(s, grid, vec, static_cast<const float *>(x), lse, pg, labels, grad_out, static_cast<float *>(out),
+                         cells, V, blank, U, divU, divTU, srows, sv);
     count_launch();
     return cudaGetLastError();
 }
